@@ -64,7 +64,13 @@ def parse():
     ap.add_argument("--no-sampling", action="store_true")
     ap.add_argument("--no-hbm", action="store_true")
     ap.add_argument("--cpu-sample-steps", type=int, default=1, help="CPU reverse steps for the sampling baseline")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned to DIR/<name>.npy (float32): its loss, a fixed seeded "
+                         "sample of the parameters it updated and, unless --no-sampling, the sampled volume")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the B200 arm's outputs; the reference arm times a batch-1 fp32 CPU step")
+    return args
 
 
 def peaks():
@@ -82,6 +88,21 @@ def peaks():
 def unet_kwargs():
     from medical_image_generation_b200 import planner
     return planner.ddpm_kwargs(list(LATENT[1:]), latent_channels=LATENT[0])
+
+
+PARAM_SAMPLE = 1 << 22   # parameters written by --dump-outputs (16 MB of float32)
+
+
+def training_outputs(model, loss) -> dict:
+    """The loss of the last training step and a fixed, seeded sample of the parameters it left behind. The parameters
+    are taken in name order, each flattened in its own index order, so the sample does not depend on memory format or
+    on how the optimiser lays out its flat buffers."""
+    import torch
+    with torch.no_grad():
+        flat = torch.cat([p.detach().reshape(-1) for _, p in sorted(model.named_parameters())])
+        idx = torch.randint(flat.numel(), (min(PARAM_SAMPLE, flat.numel()),), generator=torch.Generator().manual_seed(0))
+        params = flat[idx.sort().values.to(flat.device)].float().cpu().numpy()
+    return {"loss": loss.detach().float().cpu().numpy(), "params": params}
 
 
 def rerandomize_zero_init(module, seed=1234, std=0.02):
@@ -260,10 +281,10 @@ class ClockSampler:
 # --------------------------------------------------------------------------------------------------
 # sampling block (BASELINE config 4) and HBM-roofline block
 # --------------------------------------------------------------------------------------------------
-def sampling_block(args, dev, world, rank, sync_all, pk):
+def sampling_block(args, dev, world, rank, sync_all, pk, outputs=None):
     """One volume per rank through the public API (`DiffusionInferer.sample`): pinned-host noise -> H2D -> `sample_steps`
     reverse steps (U-Net forward + fused scheduler step, step noise drawn on the device) -> D2H of the volume.
-    Returns the `sampling` object of the JSON line (rank 0) or None."""
+    Returns the `sampling` object of the JSON line (rank 0) or None; rank 0 adds the volume to `outputs` if given."""
     import torch
     import torch.distributed as dist
     import medical_image_generation_b200 as mig
@@ -302,6 +323,8 @@ def sampling_block(args, dev, world, rank, sync_all, pk):
     del model
     if rank != 0:
         return None
+    if outputs is not None:
+        outputs["sampled_volume"] = out.float().numpy()
     ms_step = dev_ms / K
     vpm = world * 60.0 / (ms_step * 1000 / 1e3)
     tflops = SAMPLING_FLOP_PER_FORWARD / (ms_step * 1e-3) / 1e12
@@ -504,6 +527,11 @@ def run_b200(args):
     sync_all()
     w1 = time.perf_counter()
     ms = e0.elapsed_time(e1)
+    # what the last timed step returned, taken before the instrumented steps below train the model further
+    outputs = None
+    if args.dump_outputs:
+        trainer.opt.consolidate()   # collective: the sharded optimiser holds current masters only for its own slices
+        outputs = training_outputs(model, loss) if rank == 0 else None
     # per-kernel CUDA events need the Python launch path (a graph replay has no per-node events): the same step is
     # run eagerly, instrumented, directly after the timed region -- same workload, same kernels, same stream.
     prof_steps = min(args.steps, 3)
@@ -548,7 +576,7 @@ def run_b200(args):
     sampling = hbm = None
     if not args.no_sampling:
         # the training state (flat buffers, captured graph) is no longer needed: free it for the sampling model
-        sampling = sampling_block(args, dev, world, rank, sync_all, pk)
+        sampling = sampling_block(args, dev, world, rank, sync_all, pk, outputs)
     if rank == 0 and not args.no_hbm:
         hbm = hbm_block(dev, pk)
     if rank == 0:
@@ -629,6 +657,11 @@ def run_b200(args):
                 "gpu_launches": launches,
                 "clocks": clocks, "roofline": roofline, "cpu_baseline": cpu, "sampling": sampling,
                 "hbm_roofline": hbm}
+        if outputs is not None:
+            import numpy as np
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, array in outputs.items():
+                np.save(os.path.join(args.dump_outputs, name + ".npy"), array)
         print(json.dumps(line), flush=True)
     if world > 1:
         # Teardown: the captured step graph holds NCCL work; destroying the communicator with such a graph alive can

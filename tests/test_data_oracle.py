@@ -9,6 +9,7 @@ import torch
 
 from oracle import data_oracle as D
 from oracle import reference_loader as ref
+from oracle.gen_golden_checks import BBOX_PATCH, fake_task, normalized_split, random_boxes
 from oracle.gen_golden_data import DATASETS, make_case
 
 
@@ -79,29 +80,29 @@ def test_soft_augmentation_params_match_reference_golden(golden):
             assert mine == draws
 
 
-@pytest.mark.skipif(not ref.available(), reason="/root/reference not present (GPU box)")
-def test_oracle_matches_live_reference_random_boxes():
-    """Random boxes through the unmodified crop_and_pad_nd and get_bbox, live."""
-    fn = ref.data_functions()
-    rs = np.random.RandomState(11)
-    for _ in range(60):
-        shape = tuple(int(v) for v in rs.randint(1, 12, size=4))
-        img = rs.rand(*shape).astype(np.float32)
-        bbox = [[int(lo), int(lo + rs.randint(1, 14))] for lo in rs.randint(-8, 12, size=3)]
-        assert np.array_equal(D.crop_and_pad_nd(img, bbox, 0), fn["crop_and_pad_nd"](img, bbox, 0)), (shape, bbox)
-    ds = fn["MedicalDataset"]("/nonexistent/", [], 4, "training",
-                              {"patch_size": [16, 24, 24], "scaling": False, "rotation": False, "gaussian_noise": False,
-                               "gaussian_blur": False, "low_resolution": False, "brightness": False, "contrast": False,
-                               "gamma": False, "mirror": False, "dummy_2d": False}, 0.5)
-    for trial in range(40):
-        shape = tuple(int(v) for v in rs.randint(6, 60, size=3))
-        locs = {1: [tuple(int(rs.randint(s)) for s in shape) for _ in range(3)], 2: []}
-        force = bool(trial % 2)
+def test_oracle_matches_live_reference_random_boxes(golden):
+    """Random boxes through crop_and_pad_nd and get_bbox against the unmodified functions' results: stored in
+    tests/golden/reference_checks.pt, and computed live as well when the reference is present."""
+    stored = golden("reference_checks")
+    crops, trials = random_boxes()
+    fn = ref.data_functions() if ref.available() else None
+    assert len(crops) == len(stored["crops"]) == 60 and len(trials) == len(stored["bboxes"]) == 40
+    for (img, bbox), want in zip(crops, stored["crops"]):
+        assert (img.shape, bbox) == (want["shape"], want["bbox"])      # the seeded inputs are the recorded ones
+        got = D.crop_and_pad_nd(img, bbox, 0)
+        assert got.shape == want["out_shape"], bbox
+        assert hashlib.sha256(np.ascontiguousarray(got).tobytes()).hexdigest() == want["sha256"], bbox
+        if fn is not None:
+            assert np.array_equal(got, fn["crop_and_pad_nd"](img, bbox, 0)), (img.shape, bbox)
+    if fn is not None:
+        ds = fn["MedicalDataset"]("/nonexistent/", [], 4, "training", {"patch_size": list(BBOX_PATCH), **_OFF}, 0.5)
+    for (trial, shape, force, locs), want in zip(trials, stored["bboxes"]):
         np.random.seed(trial)
-        want = ds.get_bbox(shape, force, locs)
-        np.random.seed(trial)
-        got = D.get_bbox(shape, force, locs, (16, 24, 24), [0, 0, 0])
-        assert [list(map(int, v)) for v in got] == [list(map(int, v)) for v in want], (shape, force)
+        got = D.get_bbox(shape, force, locs, BBOX_PATCH, [0, 0, 0])
+        assert [list(map(int, v)) for v in got] == want, (shape, force)
+        if fn is not None:
+            np.random.seed(trial)
+            assert [list(map(int, v)) for v in ds.get_bbox(shape, force, locs)] == want, (shape, force)
 
 
 def test_affine_identity_and_transform_algebra():
@@ -254,32 +255,22 @@ def test_data_path_refuses_cpu():
     assert pkg._DESC.itemsize == 152
 
 
-def _fake_task(root, n=20, ext=".zarr"):
-    import os
-    images = os.path.join(root, "Task007_Fake", "imagesTr")
-    os.makedirs(images)
-    for i in range(n):
-        path = os.path.join(images, f"pat{i:03d}{ext}")
-        if ext == ".zarr":
-            os.makedirs(path)
-        else:
-            open(path, "wb").close()
-    return os.path.join(root, "Task007_Fake")
-
-
 @pytest.mark.parametrize("splitting", ["train-val-test", "5-fold"])
-def test_split_files_like_reference(tmp_path, monkeypatch, splitting):
+def test_split_files_like_reference(golden, tmp_path, monkeypatch, splitting):
     """create_split_files / get_data_ids (data_processing.py:34-116): 70 / 10 / 20 split or 5 folds with seed 12345, file
-    reused when present; identical to the unmodified reference functions when they are available."""
+    reused when present; identical to the unmodified reference functions' split, stored in
+    tests/golden/reference_checks.pt and computed live as well when the reference is present."""
     import json
     import os
     mine_root = tmp_path / "mine"
     mine_root.mkdir()
-    task = _fake_task(str(mine_root))
+    task = fake_task(str(mine_root))
     monkeypatch.setenv("medimgen_preprocessed", str(mine_root))
     path = pkg.create_split_files("007", splitting, "3d")
     assert os.path.dirname(path) == task
     split = json.load(open(path))
+    want = golden("reference_checks")["splits"][splitting]
+    assert normalized_split(split) == want
     names = sorted(f"pat{i:03d}" for i in range(20))
     if splitting == "train-val-test":
         assert os.path.basename(path) == "splits_train_val_test.json"
@@ -303,21 +294,18 @@ def test_split_files_like_reference(tmp_path, monkeypatch, splitting):
     if ref.available():
         ref_root = tmp_path / "ref"
         ref_root.mkdir()
-        _fake_task(str(ref_root))
+        fake_task(str(ref_root))
         monkeypatch.setenv("medimgen_preprocessed", str(ref_root))
         fn = ref.data_functions()
-        want = json.load(open(fn["create_split_files"]("007", splitting, "3d")))
+        assert normalized_split(json.load(open(fn["create_split_files"]("007", splitting, "3d")))) == want
         monkeypatch.setenv("medimgen_preprocessed", str(mine_root))
-        got = json.load(open(pkg.create_split_files("007", splitting, "3d")))
-        norm = (lambda s: {k: sorted(v) for k, v in s.items()}) if splitting == "train-val-test" else \
-            (lambda s: [{k: sorted(v) for k, v in f.items()} for f in s])
-        assert norm(got) == norm(want)
+        assert normalized_split(json.load(open(pkg.create_split_files("007", splitting, "3d")))) == want
 
 
 def test_npz_cases_are_found_when_there_is_no_zarr(tmp_path, monkeypatch):
     mine_root = tmp_path / "npz"
     mine_root.mkdir()
-    _fake_task(str(mine_root), n=10, ext=".npz")
+    fake_task(str(mine_root), n=10, ext=".npz")
     monkeypatch.setenv("medimgen_preprocessed", str(mine_root))
     import json
     split = json.load(open(pkg.create_split_files("007", "train-val-test", "3d")))

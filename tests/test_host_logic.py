@@ -192,28 +192,27 @@ def test_package_planner_matches_reference_golden(golden):
         assert planner.compute_output_size(list(size), got) == plan["out"][(size, n)]
 
 
-def test_package_planner_kwargs_match_reference_dicts():
-    """create_autoencoder_dict / create_ddpm_dict (configuration.py:821-902) run live from the reference when it is
-    present: the constructor kwargs the package planner emits must equal the reference's `vae_params` / `ddpm_params`."""
+def test_package_planner_kwargs_match_reference_dicts(golden):
+    """create_autoencoder_dict / create_ddpm_dict (configuration.py:821-902): the constructor kwargs the package planner
+    emits must equal the reference's `vae_params` / `ddpm_params`, stored in tests/golden/reference_checks.pt and, when
+    the reference is present, also computed live from it."""
     from oracle import reference_loader as ref
+    from oracle.gen_golden_checks import PLANNER_PATCHES, planner_ds_cfg
     from medical_image_generation_b200 import planner
-    if not ref.available():
-        pytest.skip("reference checkout not present on this box")
-    pf = ref.planner_functions()
-    for patch, in_ch in (([96, 96, 96], 1), ([160, 160, 128], 2), ([448, 512, 512], 1), ([64, 64], 1)):
-        nd = len(patch)
-        ds_cfg = {"median_shape": patch, "max_shape": patch if nd == 3 else [1] + patch}
-        vae = pf["create_autoencoder_dict"](ds_cfg, list(range(in_ch)), nd)
+    stored = golden("reference_checks")["planner_dicts"]
+    pf = ref.planner_functions() if ref.available() else None
+    for patch, in_ch in PLANNER_PATCHES:
+        want = stored[(tuple(patch), in_ch)]
+        if pf is not None:
+            nd = len(patch)
+            assert pf["create_autoencoder_dict"](planner_ds_cfg(patch), list(range(in_ch)), nd) == want["vae"], patch
+            assert pf["create_ddpm_dict"](planner_ds_cfg(patch), nd) == want["ddpm"], patch
         mine = planner.autoencoder_kwargs(patch, in_channels=in_ch)
-        assert set(vae) == set(mine)
-        for k, v in vae.items():
-            assert mine[k] == v, (patch, k, mine[k], v)
-        ddpm = pf["create_ddpm_dict"](ds_cfg, nd)
         latent = planner.compute_output_size(patch, mine["downsample_parameters"])
-        got = planner.ddpm_kwargs(latent, latent_channels=8)
-        assert set(ddpm) == set(got)
-        for k, v in ddpm.items():
-            assert got[k] == v, (patch, k, got[k], v)
+        for name, got in (("vae", mine), ("ddpm", planner.ddpm_kwargs(latent, latent_channels=8))):
+            assert set(got) == set(want[name])
+            for k, v in want[name].items():
+                assert got[k] == v, (patch, name, k, got[k], v)
 
 
 def test_autoencoder_initialize_covers_transposed_convs():
