@@ -3,6 +3,7 @@ by the UNMODIFIED reference and (b) the CPU oracle run live on the same seeded i
 fp32 path: 1e-4 relative; bf16 path: 2e-2 relative (BASELINE.json north_star)."""
 import pytest
 import torch
+import torch.nn.functional as F
 
 from util import BF16_TOL, FP32_TOL, graph_vs_eager, rel_err, tol_for
 
@@ -547,7 +548,8 @@ def test_cuda_graph_step_replays_correctly(golden):
 
 
 def test_ae_trainer_and_sampling_sharder(golden):
-    """AETrainer (L1 + kl_weight*KL generator step) lowers the loss; sample_volumes is seed-deterministic per volume
+    """AETrainer (L1 + kl_weight*KL generator step) lowers the loss, and its first fp32 step gives the oracle's loss and
+    gradient norm; sample_volumes is seed-deterministic per volume
     (what the N-rank sharder relies on: volume v always uses seed base+v wherever it runs)."""
     import medical_image_generation_b200 as mig
     from medical_image_generation_b200.engine import AETrainer, sample_volumes
@@ -558,6 +560,20 @@ def test_ae_trainer_and_sampling_sharder(golden):
     losses = [float(tr.step(x)) for _ in range(12)]
     assert losses[-1] < losses[0], losses
     tr.opt.close()
+    # the first step in fp32 against the oracle on the CPU: same weights, images and sampling noise
+    from oracle import torch_oracle as O
+    m32, params = _build(g, torch.float32)
+    tr32 = AETrainer(m32, lr=1e-3, kl_weight=1e-7)
+    eps = g["inputs"]["eps"]
+    loss = float(tr32.step(x, eps=eps.to(DEV)))
+    ref = {k: v.float().clone().requires_grad_(True) for k, v in params.items()}
+    recon, z_mu, z_sigma = O.ae_forward(ref, g["cfg"], g["inputs"]["x"].float(), eps)
+    ref_loss = F.l1_loss(recon, g["inputs"]["x"].float()) + 1e-7 * O.kl_loss(z_mu, z_sigma)
+    ref_loss.backward()
+    ref_norm = sum(float(p.grad.double().pow(2).sum()) for p in ref.values() if p.grad is not None) ** 0.5
+    assert abs(loss - float(ref_loss)) <= FP32_TOL * float(ref_loss), (loss, float(ref_loss))
+    assert abs(float(tr32.opt.grad_norm()) - ref_norm) <= FP32_TOL * ref_norm, (float(tr32.opt.grad_norm()), ref_norm)
+    tr32.opt.close()
     gu = golden("unet3d_aniso")
     u, _ = _build(gu, torch.float32)
     kw = dict(num_train_timesteps=1000, schedule="scaled_linear_beta", beta_start=0.0015, beta_end=0.0205)
