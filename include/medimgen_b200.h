@@ -221,6 +221,12 @@ int mig_ddpm_add_noise(int dtype, const void* x0, const void* noise, const int64
 int mig_ddpm_step(int dtype, const void* model_out, const void* x, const void* z, void* prev, void* x0_hat,
                   int64_t n, float sqrt_acp_t, float sqrt_one_minus_acp_t, float c0, float ct, float sigma,
                   int prediction, int clip, void* stream);
+/* one DDIM step (DDIMScheduler.step / reversed_step): prev = sqrt_acp_prev*clamp(x0_hat) + dir_coef*eps + sigma*z,
+ * eps derived from the UNCLIPPED x0_hat; writes the (clipped) x0_hat when non-NULL. prediction: 0 epsilon, 1 sample,
+ * 2 v_prediction. `z` may be NULL when sigma == 0 (eta == 0, and every inversion step). */
+int mig_ddim_step(int dtype, const void* model_out, const void* x, const void* z, void* prev, void* x0_hat,
+                  int64_t n, float sqrt_acp_t, float sqrt_one_minus_acp_t, float sqrt_acp_prev, float dir_coef,
+                  float sigma, int prediction, int clip, void* stream);
 
 /* ---- K16/K17: losses --------------------------------------------------------------------------- */
 /* out[0] = mean((a-b)^2) (ldm:169) or mean(|a-b|) (aetrain:414); `partials` needs 2048 floats */

@@ -8,7 +8,8 @@ a CUDA device, and raises otherwise.
 """
 from .autoencoderkl import AutoencoderKL
 from .inferers import DiffusionInferer, LatentDiffusionInferer
-from .schedulers import DDPMScheduler
+from .schedulers import DDIMScheduler, DDPMScheduler
 from .unet import DiffusionModelUNet
 
-__all__ = ["AutoencoderKL", "DiffusionModelUNet", "DDPMScheduler", "DiffusionInferer", "LatentDiffusionInferer"]
+__all__ = ["AutoencoderKL", "DiffusionModelUNet", "DDPMScheduler", "DDIMScheduler", "DiffusionInferer",
+           "LatentDiffusionInferer"]

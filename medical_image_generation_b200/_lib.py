@@ -85,6 +85,7 @@ _SIGNATURES = {
     "mig_timestep_embedding": [_p, _p, _i, _i, _i, _f, _p],
     "mig_ddpm_add_noise": [_i, _p, _p, _p, _p, _p, _i, _l, _i, _i, _p],
     "mig_ddpm_step": [_i, _p, _p, _p, _p, _p, _l, _f, _f, _f, _f, _f, _i, _i, _p],
+    "mig_ddim_step": [_i, _p, _p, _p, _p, _p, _l, _f, _f, _f, _f, _f, _i, _i, _p],
     "mig_mse_fwd": [_i, _p, _p, _p, _p, _l, _i, _p],
     "mig_mse_bwd": [_i, _p, _p, _p, _p, _l, _i, _p],
     "mig_kl_fwd": [_i, _p, _p, _p, _p, _l, _i, _p],

@@ -907,6 +907,44 @@ __global__ void __launch_bounds__(256) ddpm_step_kernel(const T* __restrict__ ep
     if (x0_out) x0_out[i] = from_f<T>(x0);
   }
 }
+
+// DDIM (Song et al.): prev = ap*clamp(x0) + dir*eps + sigma*z. Unlike ddpm_step, eps enters as its own term and is
+// derived from the UNCLIPPED x0, so the clipped and unclipped predictions are both live and no (c0, ct) pair of the
+// DDPM posterior can express it. Also serves the inversion step (sigma = 0, ap/dir of the next timestep).
+struct DdimCoef { float sa, sb, ap, dir, sigma; int prediction, clip; };
+template <typename T>
+__global__ void __launch_bounds__(256) ddim_step_kernel(const T* __restrict__ m, const T* __restrict__ x,
+                                                        const T* __restrict__ z, T* __restrict__ prev,
+                                                        T* __restrict__ x0_out, int64_t n, DdimCoef k, int vec) {
+  constexpr int V = Vec16<T>::N;
+  const int64_t nvec = vec ? n / V : 0;
+  auto f = [&](float mv, float xv, float zv, float& x0) {
+    float eps;
+    if (k.prediction == 0) { x0 = (xv - k.sb * mv) / k.sa; eps = mv; }
+    else if (k.prediction == 1) { x0 = mv; eps = (xv - k.sa * x0) / k.sb; }
+    else { x0 = k.sa * xv - k.sb * mv; eps = k.sa * mv + k.sb * xv; }
+    if (k.clip) x0 = fminf(fmaxf(x0, -1.f), 1.f);
+    return k.ap * x0 + k.dir * eps + k.sigma * zv;
+  };
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < nvec; i += (int64_t)gridDim.x * blockDim.x) {
+    Vec16<T> vm = ld16_stream(m + i * V), vx = ld16_stream(x + i * V), vz, vp, v0;
+    if (z) vz = ld16_stream(z + i * V);
+#pragma unroll
+    for (int j = 0; j < V; ++j) {
+      float x0;
+      vp.set(j, f(vm.get(j), vx.get(j), z ? vz.get(j) : 0.f, x0));
+      v0.set(j, x0);
+    }
+    st16(prev + i * V, vp);
+    if (x0_out) st16(x0_out + i * V, v0);
+  }
+  for (int64_t i = nvec * V + (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n;
+       i += (int64_t)gridDim.x * blockDim.x) {
+    float x0;
+    prev[i] = from_f<T>(f(to_f(m[i]), to_f(x[i]), z ? to_f(z[i]) : 0.f, x0));
+    if (x0_out) x0_out[i] = from_f<T>(x0);
+  }
+}
 }  // namespace mig
 
 extern "C" int mig_ddpm_add_noise(int dtype, const void* x0, const void* noise, const int64_t* timesteps,
@@ -939,6 +977,23 @@ extern "C" int mig_ddpm_step(int dtype, const void* model_out, const void* x, co
         (const TT*)model_out, (const TT*)x, (const TT*)z, (TT*)prev, (TT*)x0_hat, n, k, vec);
   });
   return check_launch("ddpm_step");
+}
+
+extern "C" int mig_ddim_step(int dtype, const void* model_out, const void* x, const void* z, void* prev, void* x0_hat,
+                             int64_t n, float sqrt_acp_t, float sqrt_one_minus_acp_t, float sqrt_acp_prev,
+                             float dir_coef, float sigma, int prediction, int clip, void* stream) {
+  if (n <= 0) return 0;
+  MIG_REQUIRE(z != nullptr || sigma == 0.f, "ddim_step: noise buffer required when sigma != 0");
+  MIG_REQUIRE(prediction >= 0 && prediction <= 2, "ddim_step: prediction must be 0, 1 or 2");
+  DdimCoef k{sqrt_acp_t, sqrt_one_minus_acp_t, sqrt_acp_prev, dir_coef, sigma, prediction, clip};
+  MIG_DISPATCH_DTYPE(dtype, TT, {
+    constexpr int V = Vec16<TT>::N;
+    int vec = aligned16(model_out) && aligned16(x) && aligned16(prev) && (!z || aligned16(z)) &&
+              (!x0_hat || aligned16(x0_hat));
+    ddim_step_kernel<TT><<<bw_grid((n + V - 1) / V, 256), 256, 0, as_stream(stream)>>>(
+        (const TT*)model_out, (const TT*)x, (const TT*)z, (TT*)prev, (TT*)x0_hat, n, k, vec);
+  });
+  return check_launch("ddim_step");
 }
 
 // ------------------------------------------------------------------------------------------------

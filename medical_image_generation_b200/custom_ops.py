@@ -5,6 +5,7 @@
     torch.ops.medimgen_b200.sdpa(q, k, v, heads, scale) -> (out, lse)          # fused flash-style attention (bf16)
     torch.ops.medimgen_b200.ddpm_add_noise(x0, noise, timesteps, alphas_cumprod, velocity) -> Tensor
     torch.ops.medimgen_b200.ddpm_step(model_output, sample, z, sqrt_acp, sqrt_1m_acp, c0, ct, sigma, prediction, clip) -> (prev, x0)
+    torch.ops.medimgen_b200.ddim_step(model_output, sample, z, sqrt_acp, sqrt_1m_acp, sqrt_acp_prev, dir_coef, sigma, prediction, clip) -> (prev, x0)
     torch.ops.medimgen_b200.mse_loss(pred, target, l1) -> Tensor
 
 BASELINE.json's north star asks for the C ABI to be "exposed as PyTorch custom ops": these are the dispatcher-visible
@@ -193,6 +194,36 @@ def _(model_output, sample, z, sqrt_acp, sqrt_one_minus_acp, c0, ct, sigma, pred
     return e, torch.empty_like(e)
 
 
+def _check_step_operands(name, model_output, sample, z):
+    if model_output.shape != sample.shape or (z is not None and z.shape != sample.shape):
+        raise RuntimeError(f"{name}: model_output {tuple(model_output.shape)}, sample {tuple(sample.shape)} and z "
+                           f"{None if z is None else tuple(z.shape)} must have one shape")
+    if sample.dtype not in (torch.float32, torch.bfloat16):
+        raise RuntimeError(f"{name}: sample must be float32 or bfloat16, got {sample.dtype}")
+
+
+@torch.library.custom_op(f"{NS}::ddim_step", mutates_args=(), device_types="cuda")
+def ddim_step(model_output: torch.Tensor, sample: torch.Tensor, z: Optional[torch.Tensor], sqrt_acp: float,
+              sqrt_one_minus_acp: float, sqrt_acp_prev: float, dir_coef: float, sigma: float, prediction: int,
+              clip: bool) -> Tuple[torch.Tensor, torch.Tensor]:
+    _check_step_operands("ddim_step", model_output, sample, z)
+    x = sample.contiguous()
+    m = model_output.to(x.dtype).contiguous()
+    zz = None if z is None else z.to(x.dtype).contiguous()
+    prev, x0 = torch.empty_like(x), torch.empty_like(x)
+    call("mig_ddim_step", ops._dt(x), ops._ptr(m), ops._ptr(x), ops._ptr(zz), ops._ptr(prev), ops._ptr(x0), x.numel(),
+         float(sqrt_acp), float(sqrt_one_minus_acp), float(sqrt_acp_prev), float(dir_coef),
+         float(sigma) if zz is not None else 0.0, int(prediction), int(clip), ops._stream())
+    return prev, x0
+
+
+@ddim_step.register_fake
+def _(model_output, sample, z, sqrt_acp, sqrt_one_minus_acp, sqrt_acp_prev, dir_coef, sigma, prediction, clip):
+    _check_step_operands("ddim_step", model_output, sample, z)
+    e = torch.empty_like(sample, memory_format=torch.contiguous_format)
+    return e, torch.empty_like(e)
+
+
 @torch.library.custom_op(f"{NS}::mse_loss", mutates_args=(), device_types="cuda")
 def mse_loss(pred: torch.Tensor, target: torch.Tensor, l1: bool) -> torch.Tensor:
     a, b = ops._pair(pred, target)
@@ -219,4 +250,4 @@ def _mse_backward(ctx, g):
 
 mse_loss.register_autograd(_mse_backward, setup_context=_mse_setup)
 
-__all__ = ["conv_nd", "group_norm", "sdpa", "ddpm_add_noise", "ddpm_step", "mse_loss"]
+__all__ = ["conv_nd", "group_norm", "sdpa", "ddpm_add_noise", "ddpm_step", "ddim_step", "mse_loss"]
