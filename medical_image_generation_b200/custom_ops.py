@@ -11,10 +11,11 @@
 BASELINE.json's north star asks for the C ABI to be "exposed as PyTorch custom ops": these are the dispatcher-visible
 entry points (schema, CUDA implementation = the C-ABI call, fake/meta implementation for shape propagation, autograd
 formula made of the C-ABI backward kernels), so the operators can be called from code that only knows `torch.ops`, be
-traced by FakeTensor-based tooling and be checked with `torch.library.opcheck`. Each implementation runs exactly the code
-of the matching `autograd.Function` in ops.py through a minimal context object -- one kernel-calling code path, two
-front ends. The nn.Modules of this package call the `autograd.Function` front end directly: it costs ~15 us less host
-time per call than a dispatcher round trip, which matters for the eager (non-CUDA-graph) step.
+traced by FakeTensor-based tooling and be checked with `torch.library.opcheck`. Each implementation calls the same
+kernel-calling functions of ops.py as the matching `autograd.Function` (`_conv_forward`, `_gn_backward`, ...) -- one
+kernel-calling code path, two front ends. The nn.Modules of this package call the `autograd.Function` front end
+directly: it costs ~15 us less host time per call than a dispatcher round trip, which matters for the eager
+(non-CUDA-graph) step.
 """
 from __future__ import annotations
 
@@ -26,18 +27,6 @@ from . import ops
 from ._lib import call
 
 NS = "medimgen_b200"
-
-
-class _Ctx:
-    """Stand-in for the autograd context object, so the registered ops reuse the Function bodies verbatim."""
-
-    def __init__(self, **kw):
-        self.saved_tensors = ()
-        self.needs_input_grad = ()
-        self.__dict__.update(kw)
-
-    def save_for_backward(self, *tensors):
-        self.saved_tensors = tensors
 
 
 def _cl_shape_like(x, shape):
@@ -54,7 +43,7 @@ def conv_nd(x: torch.Tensor, weight: torch.Tensor, bias: Optional[torch.Tensor],
         residual = ops._relayout(residual.contiguous(), x.dtype, True)
     if chan_bias is not None:
         chan_bias = chan_bias.float().contiguous()
-    return ops._ConvFn.forward(_Ctx(), x, weight, bias, chan_bias, residual, tuple(stride), tuple(padding), 0)
+    return ops._conv_forward(x, weight, bias, chan_bias, residual, tuple(stride), tuple(padding))[0]
 
 
 @conv_nd.register_fake
@@ -68,7 +57,6 @@ def _conv_setup(ctx, inputs, output):
     x, weight, bias, chan_bias, residual, stride, padding = inputs
     ctx.save_for_backward(x, weight)
     ctx.bias_ref, ctx.weight_ref = bias, weight
-    ctx.has = (bias is not None, chan_bias is not None, residual is not None)
     ctx.cfg = (tuple(stride), tuple(padding))
 
 
@@ -78,10 +66,9 @@ def _conv_backward(ctx, dy):
         x = ops._relayout(x.contiguous(), x.dtype, True)
     stride, padding = ctx.cfg
     geom, _ = ops._geom(x.shape[0], x.shape[2:], x.shape[1], weight.shape[0], weight.shape[2:], stride, padding)
-    inner = _Ctx(saved_tensors=(x, weight), geom=geom, has=ctx.has, bias_ref=ctx.bias_ref, weight_ref=ctx.weight_ref,
-                 needs_input_grad=tuple(ctx.needs_input_grad) + (False,))
-    dx, dw, db, dcb, dres, *_ = ops._ConvFn.backward(inner, dy.contiguous(memory_format=ops._mf(dy.ndim)))
-    return dx, dw, db, dcb, dres, None, None
+    grads = ops._conv_backward(x, ctx.weight_ref, ctx.bias_ref, geom, dy.contiguous(memory_format=ops._mf(dy.ndim)),
+                               *ctx.needs_input_grad[:5])
+    return (*grads, None, None)
 
 
 conv_nd.register_autograd(_conv_backward, setup_context=_conv_setup)
@@ -93,10 +80,7 @@ def group_norm(x: torch.Tensor, weight: torch.Tensor, bias: torch.Tensor, groups
                silu: bool) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
     if not ops._is_cl(x):
         x = ops._relayout(x.contiguous(), x.dtype, True)
-    ctx = _Ctx()
-    y = ops._GroupNormFn.forward(ctx, x, weight, bias, int(groups), float(eps), bool(silu))
-    _, _, _, mean, rstd = ctx.saved_tensors
-    return y, mean, rstd
+    return ops._gn_forward(x, weight, bias, int(groups), float(eps), bool(silu))
 
 
 @group_norm.register_fake
@@ -114,12 +98,10 @@ def _gn_setup(ctx, inputs, output):
 
 
 def _gn_backward(ctx, dy, _dmean, _drstd):
-    x, weight, bias, mean, rstd = ctx.saved_tensors
+    x, _, _, mean, rstd = ctx.saved_tensors
     if not ops._is_cl(x):
         x = ops._relayout(x.contiguous(), x.dtype, True)
-    inner = _Ctx(saved_tensors=(x, weight, bias, mean, rstd), cfg=ctx.cfg, refs=ctx.refs, want_colsum=False)
-    dx, dg, db, *_ = ops._GroupNormFn.backward(inner, dy)
-    return dx, dg, db, None, None, None
+    return (*ops._gn_backward(x, *ctx.refs, mean, rstd, *ctx.cfg, False, dy), None, None, None)
 
 
 group_norm.register_autograd(_gn_backward, setup_context=_gn_setup)
@@ -148,8 +130,8 @@ def _sdpa_setup(ctx, inputs, output):
 
 def _sdpa_backward(ctx, dout, _dlse):
     q, k, v, out, lse = ctx.saved_tensors
-    inner = _Ctx(saved_tensors=(q.contiguous(), k.contiguous(), v.contiguous(), out, lse), cfg=ctx.cfg)
-    dq, dk, dv, *_ = ops._FlashSdpaFn.backward(inner, dout)
+    dq, dk, dv = ops._flash_bwd(q.contiguous(), k.contiguous(), v.contiguous(), out, lse,
+                                ops._grad_in(dout, q.dtype), *ctx.cfg)
     return dq, dk, dv, None, None
 
 
@@ -227,7 +209,7 @@ def _(model_output, sample, z, sqrt_acp, sqrt_one_minus_acp, sqrt_acp_prev, dir_
 @torch.library.custom_op(f"{NS}::mse_loss", mutates_args=(), device_types="cuda")
 def mse_loss(pred: torch.Tensor, target: torch.Tensor, l1: bool) -> torch.Tensor:
     a, b = ops._pair(pred, target)
-    return ops._MseFn.forward(_Ctx(), a, b, bool(l1))
+    return ops._mse_forward(a, b, bool(l1))
 
 
 @mse_loss.register_fake
@@ -244,7 +226,7 @@ def _mse_setup(ctx, inputs, output):
 def _mse_backward(ctx, g):
     pred, target = ctx.saved_tensors
     a, b = ops._pair(pred, target)
-    da, *_ = ops._MseFn.backward(_Ctx(saved_tensors=(a, b), l1=ctx.l1), g)
+    da = ops._mse_backward(a, b, ctx.l1, g)
     return da.reshape(pred.shape).to(pred.dtype), None, None
 
 

@@ -145,6 +145,13 @@ def as_cl(x: torch.Tensor) -> torch.Tensor:
     return _relayout(x.contiguous(), x.dtype, True)
 
 
+def _grad_in(g: torch.Tensor, dtype: torch.dtype) -> torch.Tensor:
+    """An incoming gradient in the layout the backward kernels read (channels-last activations, contiguous row
+    matrices) and in `dtype`."""
+    g = as_cl(g) if g.ndim in (4, 5) else g.contiguous()
+    return g if g.dtype == dtype else g.to(dtype)
+
+
 def to_channels_last(x: torch.Tensor, dtype: torch.dtype) -> torch.Tensor:
     """(N,C,*sp) any layout/dtype -> channels-last memory in the compute dtype (differentiable)."""
     _require_cuda(x, "to_channels_last")
@@ -160,10 +167,8 @@ def from_channels_last(x: torch.Tensor, dtype: torch.dtype) -> torch.Tensor:
     return _FromChannelsLast.apply(x, dtype)
 
 
-# ----------------------------------------------------------------------------------------------
-# filter cache: compute-dtype copy of an fp32 master filter, refreshed when the parameter changes
-# ----------------------------------------------------------------------------------------------
 _PROFILE = None  # list of (kind, algorithmic flops, (Cin, Cout, out_dims, ksize), start_event, end_event) or None
+_PROFILE_SAVED = {}   # kind -> FLOPs the reference's algorithm would have spent that a folded operator did not execute
 
 
 def _profile_saved(kind: str, flops: float) -> None:
@@ -172,13 +177,10 @@ def _profile_saved(kind: str, flops: float) -> None:
 
 
 def profile_start() -> None:
-    _PROFILE_SAVED.clear()
     """bench.py: record CUDA events (on the launching stream) around every conv implicit-GEMM launch."""
     global _PROFILE
+    _PROFILE_SAVED.clear()
     _PROFILE = []
-
-
-_PROFILE_SAVED = {}   # kind -> FLOPs the reference's algorithm would have spent that a folded operator did not execute
 
 
 def profile_saved_flops() -> dict:
@@ -205,6 +207,15 @@ def _conv_call(kind, geom, name, *args):
     _PROFILE.append((kind, flops, (geom.Cin, geom.Cout, od, ks), e0, e1))
 
 
+def _conv_launch(name, which, kind, geom, dt, device, *args):
+    """Launch the implicit-GEMM entry point `name` as `name(geom, dt, *args, engine, workspace, bytes, stream)` with the
+    workspace that `mig_conv_workspace_bytes` asks for pass `which` (0 = fwd, 1 = dgrad, 2 = wgrad), profiled as `kind`.
+    `which` and `kind` name the pass the kernel serves, which is not always the entry point's own (conv-transpose,
+    upconv dgrad)."""
+    ws = _workspace(_lib.load().mig_conv_workspace_bytes(C.byref(geom), dt, which, _ENGINE), device)
+    _conv_call(kind, geom, name, C.byref(geom), dt, *args, _ENGINE, _ptr(ws), ws.numel(), _stream())
+
+
 def _deliver(param, grad):
     """Route a parameter gradient: into `param.main_grad` (flat-buffer view owned by engine.FlatAdamW) when present --
     returning None to autograd -- else hand it to autograd unchanged. `grad=None` means the kernel already accumulated
@@ -222,6 +233,25 @@ def _deliver(param, grad):
     return None
 
 
+def _grad_buf(param) -> torch.Tensor:
+    """The fp32 buffer a backward kernel ACCUMULATES `param`'s gradient into: its flat gradient buffer slot
+    (`main_grad`) when engine.FlatAdamW owns it, else a zeroed buffer of its shape and memory format. Finish with
+    `_grad_done`."""
+    mg = getattr(param, "main_grad", None)
+    if mg is not None:
+        return mg
+    return empty_cl(param.shape, torch.float32, param.device).zero_()
+
+
+def _grad_done(param, buf):
+    """What autograd receives for a gradient accumulated into `_grad_buf(param)`: None once it is in main_grad (the
+    owner is told it is ready), else the buffer."""
+    return _deliver(param, None) if getattr(param, "main_grad", None) is not None else buf
+
+
+# ----------------------------------------------------------------------------------------------
+# filter cache: compute-dtype copy of an fp32 master filter, refreshed when the parameter changes
+# ----------------------------------------------------------------------------------------------
 def _filter_for(weight: torch.Tensor, dtype: torch.dtype) -> torch.Tensor:
     if dtype == torch.bfloat16:
         shadow = getattr(weight, "_mig_shadow", None)  # bf16 copy kept current by the fused AdamW kernel
@@ -338,43 +368,84 @@ def _geom(N, in_sp, Cin, Cout, ksize, stride, pad):
     return _lib.conv_geom(N, in3, out3, Cin, Cout, k3, s3, p3), out3
 
 
-_LAST_GN_SUMS = []   # hand-over of the epilogue statistics from _ConvFn.forward to conv_nd (which tags the output)
-
-
 def _gn_split_ok(x_dtype, N, S, Cc, groups) -> bool:
     if x_dtype != torch.bfloat16 or _ENGINE == _lib.ENGINE_SIMT or not groups:
         return False
     return bool(_lib.load().mig_groupnorm_can_split(BF16, int(N), int(S), int(Cc), int(groups)))
 
 
+def _conv_forward(x, weight, bias, chan_bias, residual, stride, padding, gn_groups=0):
+    """The convolution kernel launch of conv_nd on prepared operands -> (y, geom, gn_sums). gn_sums is
+    (sums, gn_groups) when the epilogue also accumulated the GroupNorm statistics of y, else None."""
+    N, Cin = x.shape[0], x.shape[1]
+    nd = x.ndim - 2
+    Cout = weight.shape[0]
+    if weight.shape[1] != Cin:
+        raise RuntimeError(f"conv: input has {Cin} channels but the filter expects {weight.shape[1]}")
+    geom, out3 = _geom(N, x.shape[2:], Cin, Cout, weight.shape[2:], stride, padding)
+    wk = _filter_for(weight, x.dtype)
+    y = empty_cl((N, Cout, *out3[3 - nd:]), x.dtype, x.device)
+    if residual is not None and residual.shape != y.shape:
+        raise RuntimeError(f"Sizes of tensors must match: residual {tuple(residual.shape)} vs conv output "
+                           f"{tuple(y.shape)}")
+    args = (_ptr(x), _ptr(wk), _ptr(bias), _ptr(chan_bias), _ptr(residual), _ptr(y))
+    if gn_groups and _gn_split_ok(x.dtype, N, out3[0] * out3[1] * out3[2], Cout, gn_groups):
+        # the epilogue also accumulates the GroupNorm statistics of y for the norm that consumes it
+        sums = torch.empty((N, gn_groups, 2), dtype=torch.float64, device=x.device)
+        _conv_launch("mig_conv_fwd_stats", 0, "fwd", geom, _dt(x), x.device, *args, _ptr(sums), int(gn_groups))
+        return y, geom, (sums, int(gn_groups))
+    _conv_launch("mig_conv_fwd", 0, "fwd", geom, _dt(x), x.device, *args)
+    return y, geom, None
+
+
+def _conv_backward(x, weight, bias, geom, dy, want_dx, want_dw, want_db, want_dcb, want_dres):
+    """Gradients (dx, dw, db, dcb, dres) of _conv_forward; those not wanted are None. weight / bias are the parameter
+    objects (they carry main_grad and the bf16 shadow)."""
+    # per-(n, c) column sums of dy, when the GroupNorm that consumed this conv's output computed them in its own
+    # backward (ops._GroupNormFn): they ARE the time-embedding gradient, and summed over n the bias gradient
+    colsum = getattr(dy, "_mig_colsum", None)
+    if colsum is not None and tuple(colsum.shape) != (dy.shape[0], dy.shape[1]):
+        colsum = None
+    dy = _grad_in(dy, x.dtype)
+    dt = _dt(x)
+    dx = dw = db = dcb = dres = None
+    if want_dx:
+        wk = _filter_for(weight, x.dtype)
+        dx = torch.empty_like(x)
+        _conv_launch("mig_conv_dgrad", 1, "dgrad", geom, dt, x.device, _ptr(dy), _ptr(wk), _ptr(dx))
+    if want_dw or want_db:
+        # the kernels ACCUMULATE: straight into the flat gradient buffer when the engine owns the parameter
+        dw_buf = _grad_buf(weight) if want_dw else None
+        db_buf = _grad_buf(bias) if want_db else None
+        db_arg = db_buf
+        if want_db and colsum is not None:   # bias gradient = sum over samples of the ready-made column sums
+            call("mig_colsum", F32, _ptr(colsum), _ptr(db_buf), colsum.shape[0], colsum.shape[1], 1, _stream())
+            db_arg = None
+        if want_dw or db_arg is not None:
+            _conv_launch("mig_conv_wgrad", 2, "wgrad", geom, dt, x.device, _ptr(x), _ptr(dy), _ptr(dw_buf),
+                         _ptr(db_arg))
+        if want_dw:
+            dw = _grad_done(weight, dw_buf)
+        if want_db:
+            db = _grad_done(bias, db_buf)
+    if want_dcb:
+        N, Cout = dy.shape[0], dy.shape[1]
+        if colsum is not None:
+            dcb = colsum
+        else:
+            dcb = torch.empty((N, Cout), dtype=torch.float32, device=dy.device)
+            call("mig_chan_bias_bwd", dt, _ptr(dy), _ptr(dcb), N, dy.numel() // (N * Cout), Cout, _stream())
+    if want_dres:
+        dres = dy
+    return dx, dw, db, dcb, dres
+
+
 class _ConvFn(Function):
     @staticmethod
     def forward(ctx, x, weight, bias, chan_bias, residual, stride, padding, gn_groups=0):
-        N, Cin = x.shape[0], x.shape[1]
-        nd = x.ndim - 2
-        Cout = weight.shape[0]
-        if weight.shape[1] != Cin:
-            raise RuntimeError(f"conv: input has {Cin} channels but the filter expects {weight.shape[1]}")
-        geom, out3 = _geom(N, x.shape[2:], Cin, Cout, weight.shape[2:], stride, padding)
-        wk = _filter_for(weight, x.dtype)
-        y = empty_cl((N, Cout, *out3[3 - nd:]), x.dtype, x.device)
-        if residual is not None and residual.shape != y.shape:
-            raise RuntimeError(f"Sizes of tensors must match: residual {tuple(residual.shape)} vs conv output "
-                               f"{tuple(y.shape)}")
-        dt = _dt(x)
-        need = _lib.load().mig_conv_workspace_bytes(C.byref(geom), dt, 0, _ENGINE)
-        ws = _workspace(need, x.device)
-        if gn_groups and _gn_split_ok(x.dtype, N, out3[0] * out3[1] * out3[2], Cout, gn_groups):
-            # the epilogue also accumulates the GroupNorm statistics of y for the norm that consumes it
-            sums = torch.empty((N, gn_groups, 2), dtype=torch.float64, device=x.device)
-            _conv_call("fwd", geom, "mig_conv_fwd_stats", C.byref(geom), dt, _ptr(x), _ptr(wk), _ptr(bias), _ptr(chan_bias),
-                       _ptr(residual), _ptr(y), _ptr(sums), int(gn_groups), _ENGINE, _ptr(ws), ws.numel(), _stream())
-            _LAST_GN_SUMS.append((sums, int(gn_groups)))
-        else:
-            _conv_call("fwd", geom, "mig_conv_fwd", C.byref(geom), dt, _ptr(x), _ptr(wk), _ptr(bias), _ptr(chan_bias), _ptr(residual),
-                 _ptr(y), _ENGINE, _ptr(ws), ws.numel(), _stream())
-        ctx.geom = geom
-        ctx.has = (bias is not None, chan_bias is not None, residual is not None)
+        y, ctx.geom, gn_sums = _conv_forward(x, weight, bias, chan_bias, residual, stride, padding, gn_groups)
+        if gn_sums is not None:
+            y._mig_gn_sums = gn_sums   # Function.apply hands the caller this very tensor object, attribute included
         ctx.bias_ref, ctx.weight_ref = bias, weight  # the Parameter objects (carry main_grad / shadow attributes)
         ctx.save_for_backward(x, weight)
         return y
@@ -382,62 +453,8 @@ class _ConvFn(Function):
     @staticmethod
     def backward(ctx, dy):
         x, _ = ctx.saved_tensors
-        weight = ctx.weight_ref
-        geom = ctx.geom
-        # per-(n, c) column sums of dy, when the GroupNorm that consumed this conv's output computed them in its own
-        # backward (ops._GroupNormFn): they ARE the time-embedding gradient, and summed over n the bias gradient
-        colsum = getattr(dy, "_mig_colsum", None)
-        if colsum is not None and tuple(colsum.shape) != (dy.shape[0], dy.shape[1]):
-            colsum = None
-        dy = as_cl(dy)
-        if dy.dtype != x.dtype:
-            dy = dy.to(x.dtype)
-        dt = _dt(x)
-        lib = _lib.load()
-        dx = dw = db = dcb = dres = None
-        if ctx.needs_input_grad[0]:
-            wk = _filter_for(weight, x.dtype)
-            dx = torch.empty_like(x)
-            need = lib.mig_conv_workspace_bytes(C.byref(geom), dt, 1, _ENGINE)
-            ws = _workspace(need, x.device)
-            _conv_call("dgrad", geom, "mig_conv_dgrad", C.byref(geom), dt, _ptr(dy), _ptr(wk), _ptr(dx), _ENGINE, _ptr(ws), ws.numel(),
-                 _stream())
-        want_w, want_b = ctx.needs_input_grad[1], ctx.has[0] and ctx.needs_input_grad[2]
-        if want_w or want_b:
-            bias = ctx.bias_ref
-            weight = ctx.weight_ref
-            w_main = getattr(weight, "main_grad", None) if want_w else None
-            b_main = getattr(bias, "main_grad", None) if want_b else None
-            dw_buf = db_buf = None
-            if want_w:
-                dw_buf = w_main if w_main is not None else empty_cl(weight.shape, torch.float32, x.device).zero_()
-            if want_b:
-                db_buf = b_main if b_main is not None else torch.zeros(weight.shape[0], dtype=torch.float32,
-                                                                     device=x.device)
-            need = lib.mig_conv_workspace_bytes(C.byref(geom), dt, 2, _ENGINE)
-            ws = _workspace(need, x.device)
-            # the kernels ACCUMULATE: straight into the flat gradient buffer when the engine owns the parameter
-            db_arg = db_buf
-            if want_b and colsum is not None:   # bias gradient = sum over samples of the ready-made column sums
-                call("mig_colsum", F32, _ptr(colsum), _ptr(db_buf), colsum.shape[0], colsum.shape[1], 1, _stream())
-                db_arg = None
-            if want_w or db_arg is not None:
-                _conv_call("wgrad", geom, "mig_conv_wgrad", C.byref(geom), dt, _ptr(x), _ptr(dy), _ptr(dw_buf), _ptr(db_arg),
-                           _ENGINE, _ptr(ws), ws.numel(), _stream())
-            if want_w:
-                dw = _deliver(weight, None) if w_main is not None else dw_buf
-            if want_b:
-                db = _deliver(bias, None) if b_main is not None else db_buf
-        if ctx.has[1] and ctx.needs_input_grad[3]:
-            N, Cout = dy.shape[0], dy.shape[1]
-            if colsum is not None:
-                dcb = colsum
-            else:
-                dcb = torch.empty((N, Cout), dtype=torch.float32, device=dy.device)
-                call("mig_chan_bias_bwd", dt, _ptr(dy), _ptr(dcb), N, dy.numel() // (N * Cout), Cout, _stream())
-        if ctx.has[2] and ctx.needs_input_grad[4]:
-            dres = dy
-        return dx, dw, db, dcb, dres, None, None, None
+        return (*_conv_backward(x, ctx.weight_ref, ctx.bias_ref, ctx.geom, dy, *ctx.needs_input_grad[:5]), None, None,
+                None)
 
 
 def conv_nd(x, weight, bias=None, stride=1, padding=0, chan_bias=None, residual=None, gn_groups=0):
@@ -463,11 +480,7 @@ def conv_nd(x, weight, bias=None, stride=1, padding=0, chan_bias=None, residual=
         chan_bias = chan_bias.float().contiguous()
     if residual is not None and (not _is_cl(residual) or residual.dtype != x.dtype):
         residual = to_channels_last(residual, x.dtype)
-    del _LAST_GN_SUMS[:]
-    y = _ConvFn.apply(x, weight, bias, chan_bias, residual, s, p, int(gn_groups or 0))
-    if _LAST_GN_SUMS:
-        y._mig_gn_sums = _LAST_GN_SUMS.pop()
-    return y
+    return _ConvFn.apply(x, weight, bias, chan_bias, residual, s, p, int(gn_groups or 0))
 
 
 class _ConvTransposeFn(Function):
@@ -495,10 +508,7 @@ class _ConvTransposeFn(Function):
         wk = _filter_for(weight, x.dtype)
         y = empty_cl((N, Cout, *out_sp), x.dtype, x.device)
         dt = _dt(x)
-        need = _lib.load().mig_conv_workspace_bytes(C.byref(geom), dt, 1, _ENGINE)
-        ws = _workspace(need, x.device)
-        _conv_call("dgrad", geom, "mig_conv_dgrad", C.byref(geom), dt, _ptr(x), _ptr(wk), _ptr(y), _ENGINE, _ptr(ws),
-                   ws.numel(), _stream())
+        _conv_launch("mig_conv_dgrad", 1, "dgrad", geom, dt, x.device, _ptr(x), _ptr(wk), _ptr(y))
         if bias is not None:
             call("mig_add_channel_bias", dt, _ptr(y), _ptr(bias), _ptr(y), y.numel() // Cout, Cout, _stream())
         ctx.geom = geom
@@ -510,34 +520,23 @@ class _ConvTransposeFn(Function):
     def backward(ctx, dy):
         x, _ = ctx.saved_tensors
         weight, bias, geom = ctx.weight_ref, ctx.bias_ref, ctx.geom
-        dy = as_cl(dy)
-        if dy.dtype != x.dtype:
-            dy = dy.to(x.dtype)
+        dy = _grad_in(dy, x.dtype)
         dt = _dt(x)
-        lib = _lib.load()
         dx = dw = db = None
         if ctx.needs_input_grad[0]:
             wk = _filter_for(weight, x.dtype)
             dx = torch.empty_like(x)
-            need = lib.mig_conv_workspace_bytes(C.byref(geom), dt, 0, _ENGINE)
-            ws = _workspace(need, x.device)
-            _conv_call("fwd", geom, "mig_conv_fwd", C.byref(geom), dt, _ptr(dy), _ptr(wk), None, None, None, _ptr(dx),
-                       _ENGINE, _ptr(ws), ws.numel(), _stream())
+            _conv_launch("mig_conv_fwd", 0, "fwd", geom, dt, x.device, _ptr(dy), _ptr(wk), None, None, None, _ptr(dx))
         if ctx.needs_input_grad[1]:
-            w_main = getattr(weight, "main_grad", None)
-            dw_buf = w_main if w_main is not None else empty_cl(weight.shape, torch.float32, x.device).zero_()
-            need = lib.mig_conv_workspace_bytes(C.byref(geom), dt, 2, _ENGINE)
-            ws = _workspace(need, x.device)
+            dw_buf = _grad_buf(weight)
             # underlying convolution: input = dy (of this op), output gradient = x (of this op)
-            _conv_call("wgrad", geom, "mig_conv_wgrad", C.byref(geom), dt, _ptr(dy), _ptr(x), _ptr(dw_buf), None, _ENGINE,
-                       _ptr(ws), ws.numel(), _stream())
-            dw = _deliver(weight, None) if w_main is not None else dw_buf
-        if bias is not None and ctx.needs_input_grad[2]:
-            b_main = getattr(bias, "main_grad", None)
+            _conv_launch("mig_conv_wgrad", 2, "wgrad", geom, dt, x.device, _ptr(dy), _ptr(x), _ptr(dw_buf), None)
+            dw = _grad_done(weight, dw_buf)
+        if ctx.needs_input_grad[2]:
+            db_buf = _grad_buf(bias)
             Cout = dy.shape[1]
-            db_buf = b_main if b_main is not None else torch.zeros(Cout, dtype=torch.float32, device=x.device)
             call("mig_colsum", dt, _ptr(dy), _ptr(db_buf), dy.numel() // Cout, Cout, 1, _stream())
-            db = _deliver(bias, None) if b_main is not None else db_buf
+            db = _grad_done(bias, db_buf)
         return dx, dw, db, None, None, None
 
 
@@ -559,18 +558,11 @@ class _LinearFn(Function):
         rows, K = x.shape
         O = weight.shape[0]
         geom, _ = _geom(1, (1, 1, rows), K, O, (1, 1, 1), (1, 1, 1), (0, 0, 0))
-        wk = weight.detach()
-        if wk.dtype != x.dtype:
-            wk = _filter_for(weight, x.dtype)
-        wk = wk.contiguous()
+        wk = _filter_for(weight, x.dtype)
         y = torch.empty((rows, O), dtype=x.dtype, device=x.device)
-        dt = _dt(x)
-        need = _lib.load().mig_conv_workspace_bytes(C.byref(geom), dt, 0, _ENGINE)
-        ws = _workspace(need, x.device)
-        _conv_call("fwd", geom, "mig_conv_fwd", C.byref(geom), dt, _ptr(x), _ptr(wk), _ptr(bias), None, None, _ptr(y), _ENGINE, _ptr(ws),
-             ws.numel(), _stream())
+        _conv_launch("mig_conv_fwd", 0, "fwd", geom, _dt(x), x.device, _ptr(x), _ptr(wk), _ptr(bias), None, None,
+                     _ptr(y))
         ctx.geom = geom
-        ctx.has_bias = bias is not None
         ctx.bias_ref, ctx.weight_ref = bias, weight
         ctx.save_for_backward(x, weight)
         return y
@@ -578,44 +570,24 @@ class _LinearFn(Function):
     @staticmethod
     def backward(ctx, dy):
         x, _ = ctx.saved_tensors
-        weight = ctx.weight_ref
-        geom = ctx.geom
-        dy = dy.contiguous()
-        if dy.dtype != x.dtype:
-            dy = dy.to(x.dtype)
+        weight, bias, geom = ctx.weight_ref, ctx.bias_ref, ctx.geom
+        dy = _grad_in(dy, x.dtype)
         dt = _dt(x)
-        lib = _lib.load()
         dx = dw = db = None
         if ctx.needs_input_grad[0]:
-            wk = weight.detach()
-            if wk.dtype != x.dtype:
-                wk = _filter_for(weight, x.dtype)
-            wk = wk.contiguous()
+            wk = _filter_for(weight, x.dtype)
             dx = torch.empty_like(x)
-            need = lib.mig_conv_workspace_bytes(C.byref(geom), dt, 1, _ENGINE)
-            ws = _workspace(need, x.device)
-            _conv_call("dgrad", geom, "mig_conv_dgrad", C.byref(geom), dt, _ptr(dy), _ptr(wk), _ptr(dx), _ENGINE, _ptr(ws), ws.numel(),
-                 _stream())
-        want_w, want_b = ctx.needs_input_grad[1], ctx.has_bias and ctx.needs_input_grad[2]
+            _conv_launch("mig_conv_dgrad", 1, "dgrad", geom, dt, x.device, _ptr(dy), _ptr(wk), _ptr(dx))
+        want_w, want_b = ctx.needs_input_grad[1], ctx.needs_input_grad[2]
         if want_w or want_b:
-            bias = ctx.bias_ref
-            w_main = getattr(weight, "main_grad", None) if want_w else None
-            b_main = getattr(bias, "main_grad", None) if want_b else None
-            dw_buf = db_buf = None
+            dw_buf = _grad_buf(weight) if want_w else None
+            db_buf = _grad_buf(bias) if want_b else None
+            _conv_launch("mig_conv_wgrad", 2, "wgrad", geom, dt, x.device, _ptr(x), _ptr(dy), _ptr(dw_buf),
+                         _ptr(db_buf))
             if want_w:
-                dw_buf = w_main if w_main is not None else torch.zeros(weight.shape, dtype=torch.float32,
-                                                                     device=x.device)
+                dw = _grad_done(weight, dw_buf)
             if want_b:
-                db_buf = b_main if b_main is not None else torch.zeros(weight.shape[0], dtype=torch.float32,
-                                                                     device=x.device)
-            need = lib.mig_conv_workspace_bytes(C.byref(geom), dt, 2, _ENGINE)
-            ws = _workspace(need, x.device)
-            _conv_call("wgrad", geom, "mig_conv_wgrad", C.byref(geom), dt, _ptr(x), _ptr(dy), _ptr(dw_buf), _ptr(db_buf), _ENGINE, _ptr(ws),
-                 ws.numel(), _stream())
-            if want_w:
-                dw = _deliver(weight, None) if w_main is not None else dw_buf
-            if want_b:
-                db = _deliver(bias, None) if b_main is not None else db_buf
+                db = _grad_done(bias, db_buf)
         return dx, dw, db
 
 
@@ -652,37 +624,27 @@ class _TembProjAllFn(Function):
         ws, bs = ctx.refs
         n = len(ws)
         rows, K = x.shape
-        keep, dy_p, dw_p, db_p, dw_new, db_new = [], [], [], [], [None] * n, [None] * n
+        keep, dw_b, db_b = [], [None] * n, [None] * n
         for i in range(n):
-            g = grads[i]
-            if g is None:        # this layer received no gradient: the kernels skip it (null dy)
-                dy_p.append(None); dw_p.append(None); db_p.append(None)
+            if grads[i] is None:     # this layer received no gradient: the kernels skip it (null dy)
+                keep.append(None)
                 continue
-            g = g.float().contiguous()
-            keep.append(g)
-            dy_p.append(g.data_ptr())
-            wm = getattr(ws[i], "main_grad", None)
-            if wm is None:
-                dw_new[i] = wm = torch.zeros_like(wt[i])
-            dw_p.append(wm.data_ptr())
-            if bs[i] is None:
-                db_p.append(None)
-            else:
-                bm = getattr(bs[i], "main_grad", None)
-                if bm is None:
-                    db_new[i] = bm = torch.zeros(wt[i].shape[0], dtype=torch.float32, device=x.device)
-                db_p.append(bm.data_ptr())
+            keep.append(grads[i].float().contiguous())
+            dw_b[i] = _grad_buf(ws[i])
+            if bs[i] is not None:
+                db_b[i] = _grad_buf(bs[i])
         dx = torch.empty_like(x) if ctx.needs_input_grad[0] else None
         PA, IA = C.c_void_p * n, C.c_int32 * n
-        call("mig_temb_proj_all_bwd", _ptr(x), PA(*[w.data_ptr() for w in wt]), PA(*dy_p), PA(*dw_p), PA(*db_p), _ptr(dx),
+        ptrs = lambda ts: PA(*[None if t is None else t.data_ptr() for t in ts])  # noqa: E731
+        call("mig_temb_proj_all_bwd", _ptr(x), ptrs(wt), ptrs(keep), ptrs(dw_b), ptrs(db_b), _ptr(dx),
              IA(*[w.shape[0] for w in wt]), n, rows, K, _stream())
         out = [dx]
         for i in range(n):
-            if dy_p[i] is None:
+            if keep[i] is None:
                 out += [None, None]
                 continue
-            out.append(dw_new[i] if dw_new[i] is not None else _deliver(ws[i], None))
-            out.append(None if bs[i] is None else (db_new[i] if db_new[i] is not None else _deliver(bs[i], None)))
+            out.append(_grad_done(ws[i], dw_b[i]))
+            out.append(None if bs[i] is None else _grad_done(bs[i], db_b[i]))
         return tuple(out)
 
 
@@ -704,7 +666,8 @@ def temb_projections(x, linears):
 # ----------------------------------------------------------------------------------------------
 # GroupNorm (+SiLU), LayerNorm, SiLU
 # ----------------------------------------------------------------------------------------------
-def _gn_forward(ctx, x, gamma, beta, groups, eps, silu):
+def _gn_forward(x, gamma, beta, groups, eps, silu):
+    """GroupNorm (+SiLU) of channels-last x -> (y, mean, rstd)."""
     N, Cc = x.shape[0], x.shape[1]
     S = x.numel() // (N * Cc)
     y = torch.empty_like(x)
@@ -720,38 +683,30 @@ def _gn_forward(ctx, x, gamma, beta, groups, eps, silu):
         ws = _workspace(need, x.device)
         call("mig_groupnorm_fwd", _dt(x), _ptr(x), _ptr(gamma), _ptr(beta), _ptr(y), _ptr(mean), _ptr(rstd), N, S, Cc,
              groups, float(eps), int(silu), _ptr(ws), ws.numel(), _stream())
-    ctx.save_for_backward(x, gamma, beta, mean, rstd)
-    ctx.cfg = (groups, silu)
-    ctx.refs = (gamma, beta)
-    ctx.want_colsum = bool(getattr(x, "_mig_sole_consumer_gn", False))
-    return y
+    return y, mean, rstd
 
 
-def _gn_backward(ctx, dy, dskip=None):
-    """dskip: the gradient that reaches x through the block's skip path (x also feeds the residual add / skip conv): it is
-    added inside the GroupNorm backward kernel instead of by a separate accumulation pass."""
-    x, gamma, beta, mean, rstd = ctx.saved_tensors
-    groups, silu = ctx.cfg
+def _gn_backward(x, gamma, beta, mean, rstd, groups, silu, want_colsum, dy, dskip=None):
+    """-> (dx, dgamma, dbeta). gamma / beta are the parameter objects (they carry main_grad).
+    dskip: the gradient that reaches x through the block's skip path (x also feeds the residual add / skip conv): it is
+    added inside the GroupNorm backward kernel instead of by a separate accumulation pass.
+    want_colsum: x is the output of a convolution that only this norm consumes; hand that convolution's backward the
+    column sums of dx (`_mig_colsum`)."""
     N, Cc = x.shape[0], x.shape[1]
     S = x.numel() // (N * Cc)
     if dy is None:   # the normalised branch got no gradient: only the skip path contributes
         return (None if dskip is None else as_cl(dskip)), None, None
-    dy = as_cl(dy)
-    if dy.dtype != x.dtype:
-        dy = dy.to(x.dtype)
+    dy = _grad_in(dy, x.dtype)
     if dskip is not None:
-        dskip = as_cl(dskip)
-        if dskip.dtype != x.dtype:
-            dskip = dskip.to(x.dtype)
+        dskip = _grad_in(dskip, x.dtype)
     dx = torch.empty_like(x)
-    gref, bref = ctx.refs
-    g_main, b_main = getattr(gref, "main_grad", None), getattr(bref, "main_grad", None)
+    g_main, b_main = getattr(gamma, "main_grad", None), getattr(beta, "main_grad", None)
     into_main = g_main is not None and b_main is not None     # accumulate straight into the flat gradient buffer
     dgamma = g_main if into_main else torch.empty_like(gamma)
     dbeta = b_main if into_main else torch.empty_like(beta)
     need = _lib.load().mig_groupnorm_workspace_bytes(N, S, Cc, groups)
     ws = _workspace(need, x.device)
-    colsum = torch.empty((N, Cc), dtype=torch.float32, device=x.device) if (ctx.want_colsum and dskip is None) else None
+    colsum = torch.empty((N, Cc), dtype=torch.float32, device=x.device) if (want_colsum and dskip is None) else None
     call("mig_groupnorm_bwd", _dt(x), _ptr(x), _ptr(dy), _ptr(gamma), _ptr(beta), _ptr(mean), _ptr(rstd), _ptr(dx),
          _ptr(dgamma), _ptr(dbeta), _ptr(colsum), _ptr(dskip), int(into_main), N, S, Cc, groups, int(silu), _ptr(ws),
          ws.numel(), _stream())
@@ -761,19 +716,23 @@ def _gn_backward(ctx, dy, dskip=None):
         # (several consumers -> accumulated gradient) the attribute is simply absent and the conv sums dy itself
         dx._mig_colsum = colsum
     if into_main:
-        return dx, _deliver(gref, None), _deliver(bref, None)
-    return dx, _deliver(gref, dgamma), _deliver(bref, dbeta)
+        return dx, _deliver(gamma, None), _deliver(beta, None)
+    return dx, _deliver(gamma, dgamma), _deliver(beta, dbeta)
 
 
 class _GroupNormFn(Function):
     @staticmethod
     def forward(ctx, x, gamma, beta, groups, eps, silu):
-        return _gn_forward(ctx, x, gamma, beta, groups, eps, silu)
+        y, mean, rstd = _gn_forward(x, gamma, beta, groups, eps, silu)
+        ctx.save_for_backward(x, gamma, beta, mean, rstd)
+        ctx.refs = (gamma, beta)   # the Parameter objects (carry main_grad)
+        ctx.cfg = (groups, silu, bool(getattr(x, "_mig_sole_consumer_gn", False)))
+        return y
 
     @staticmethod
     def backward(ctx, dy):
-        dx, dg, db = _gn_backward(ctx, dy)
-        return dx, dg, db, None, None, None
+        x, _, _, mean, rstd = ctx.saved_tensors
+        return (*_gn_backward(x, *ctx.refs, mean, rstd, *ctx.cfg, dy), None, None, None)
 
 
 class _GroupNormSkipFn(Function):
@@ -783,12 +742,16 @@ class _GroupNormSkipFn(Function):
 
     @staticmethod
     def forward(ctx, x, gamma, beta, groups, eps, silu):
-        return _gn_forward(ctx, x, gamma, beta, groups, eps, silu), x.view_as(x)
+        y, mean, rstd = _gn_forward(x, gamma, beta, groups, eps, silu)
+        ctx.save_for_backward(x, gamma, beta, mean, rstd)
+        ctx.refs = (gamma, beta)   # the Parameter objects (carry main_grad)
+        ctx.cfg = (groups, silu, bool(getattr(x, "_mig_sole_consumer_gn", False)))
+        return y, x.view_as(x)
 
     @staticmethod
     def backward(ctx, dy, dskip):
-        dx, dg, db = _gn_backward(ctx, dy, dskip)
-        return dx, dg, db, None, None, None
+        x, _, _, mean, rstd = ctx.saved_tensors
+        return (*_gn_backward(x, *ctx.refs, mean, rstd, *ctx.cfg, dy, dskip), None, None, None)
 
 
 def group_norm(x, gamma, beta, groups: int, eps: float, silu: bool = False, with_skip: bool = False):
@@ -1037,9 +1000,6 @@ def upsample_nearest(x, factors):
 
 
 # ----------------------------------------------------------------------------------------------
-# attention core: softmax(scale * Q K^T) V with heads inside the channel dim (unet:406-416)
-# ----------------------------------------------------------------------------------------------
-# ----------------------------------------------------------------------------------------------
 # nearest upsample folded into the convolution that follows it (K8; unet:576-584, ae:97-106)
 # ----------------------------------------------------------------------------------------------
 _UPCONV = os.environ.get("MIG_UPCONV", "auto")    # auto | always | never (A/B switch and tests)
@@ -1138,11 +1098,9 @@ class _UpConvFn(Function):
         else:
             yc = torch.empty(len(classes) * per_class, dtype=x.dtype, device=x.device)
             for ci, (geom, goff) in enumerate(geoms):
-                need = lib.mig_conv_workspace_bytes(C.byref(geom), dt, 0, _ENGINE)
-                ws = _workspace(need, x.device)
-                _conv_call("fwd", geom, "mig_conv_fwd", C.byref(geom), dt, _ptr(x),
-                           C.c_void_p(folded.data_ptr() + 2 * goff), _ptr(bias), None, None,
-                           C.c_void_p(yc.data_ptr() + 2 * ci * per_class), _ENGINE, _ptr(ws), ws.numel(), _stream())
+                _conv_launch("mig_conv_fwd", 0, "fwd", geom, dt, x.device, _ptr(x),
+                             C.c_void_p(folded.data_ptr() + 2 * goff), _ptr(bias), None, None,
+                             C.c_void_p(yc.data_ptr() + 2 * ci * per_class))
             call("mig_class_interleave", dt, _ptr(yc), _ptr(y), N, I3(*low3), ff, Cout, 0, _stream())
         ref = 2.0 * N * math.prod(low3) * math.prod(f3) * Cout * Cin * math.prod(k3)      # the reference's k^n taps
         _profile_saved("fwd", ref - sum(2.0 * N * math.prod(low3) * Cout * Cin * math.prod(g.ksize) for g, _ in geoms))
@@ -1160,9 +1118,7 @@ class _UpConvFn(Function):
         I3 = C.c_int32 * 3
         kk, ff, pp = I3(*k3), I3(*f3), I3(*p3)
         lib = _lib.load()
-        dy = as_cl(dy)
-        if dy.dtype != x.dtype:
-            dy = dy.to(x.dtype)
+        dy = _grad_in(dy, x.dtype)
         dt = _dt(x)
         dx = dw = db = None
         if ctx.needs_input_grad[0]:
@@ -1174,40 +1130,29 @@ class _UpConvFn(Function):
             geom = _lib.conv_geom(N, full3, low3, Cout, Cin, [f3[i] + k3[i] - 1 for i in range(3)], f3,
                                   [k3[i] - 1 - p3[i] for i in range(3)])
             dx = torch.empty_like(x)
-            need = lib.mig_conv_workspace_bytes(C.byref(geom), dt, 0, _ENGINE)
-            ws = _workspace(need, x.device)
-            _conv_call("dgrad", geom, "mig_conv_fwd", C.byref(geom), dt, _ptr(dy), _ptr(wd), None, None, None, _ptr(dx),
-                       _ENGINE, _ptr(ws), ws.numel(), _stream())
+            _conv_launch("mig_conv_fwd", 0, "dgrad", geom, dt, x.device, _ptr(dy), _ptr(wd), None, None, None, _ptr(dx))
             ref = 2.0 * N * math.prod(full3) * Cout * Cin * math.prod(k3)
             _profile_saved("dgrad", ref - 2.0 * N * math.prod(low3) * Cout * Cin * math.prod(geom.ksize))
-        want_w, want_b = ctx.needs_input_grad[1], bias is not None and ctx.needs_input_grad[2]
+        want_w, want_b = ctx.needs_input_grad[1], ctx.needs_input_grad[2]
         if want_w or want_b:
-            w_main = getattr(weight, "main_grad", None) if want_w else None
-            b_main = getattr(bias, "main_grad", None) if want_b else None
-            dw_buf = db_buf = None
-            if want_w:
-                dw_buf = w_main if w_main is not None else empty_cl(weight.shape, torch.float32, x.device).zero_()
-            if want_b:
-                db_buf = b_main if b_main is not None else torch.zeros(Cout, dtype=torch.float32, device=x.device)
+            dw_buf = _grad_buf(weight) if want_w else None
+            db_buf = _grad_buf(bias) if want_b else None
             # dy split into its residue classes (contiguous low-resolution tensors), one wgrad per class into the folded
             # layout, then unfolded onto the k^n taps; the bias gradient rides on the class wgrads
             dyc = torch.empty(len(geoms) * per_class, dtype=x.dtype, device=x.device)
             call("mig_class_interleave", dt, _ptr(dy), _ptr(dyc), N, I3(*low3), ff, Cout, 1, _stream())
             dwc = torch.zeros(folded_elems, dtype=torch.float32, device=x.device) if want_w else None
             for ci, (geom, off) in enumerate(geoms):
-                need = lib.mig_conv_workspace_bytes(C.byref(geom), dt, 2, _ENGINE)
-                ws = _workspace(need, x.device)
-                _conv_call("wgrad", geom, "mig_conv_wgrad", C.byref(geom), dt, _ptr(x),
-                           C.c_void_p(dyc.data_ptr() + 2 * ci * per_class),
-                           C.c_void_p(dwc.data_ptr() + 4 * off) if want_w else None, _ptr(db_buf), _ENGINE, _ptr(ws),
-                           ws.numel(), _stream())
+                _conv_launch("mig_conv_wgrad", 2, "wgrad", geom, dt, x.device, _ptr(x),
+                             C.c_void_p(dyc.data_ptr() + 2 * ci * per_class),
+                             C.c_void_p(dwc.data_ptr() + 4 * off) if want_w else None, _ptr(db_buf))
             ref = 2.0 * N * math.prod(low3) * math.prod(f3) * Cout * Cin * math.prod(k3)
             _profile_saved("wgrad", ref - sum(2.0 * N * math.prod(low3) * Cout * Cin * math.prod(g.ksize) for g, _ in geoms))
             if want_w:
                 call("mig_upconv_unfold_wgrad", _ptr(dwc), _ptr(dw_buf), Cout, Cin, kk, ff, pp, _stream())
-                dw = _deliver(weight, None) if w_main is not None else dw_buf
+                dw = _grad_done(weight, dw_buf)
             if want_b:
-                db = _deliver(bias, None) if b_main is not None else db_buf
+                db = _grad_done(bias, db_buf)
         return dx, dw, db, None, None
 
 
@@ -1226,6 +1171,9 @@ def upsample_conv_nd(x, weight, bias, factors, padding):
     return _UpConvFn.apply(x, weight, bias, fi, tuple(int(v) for v in p))
 
 
+# ----------------------------------------------------------------------------------------------
+# attention core: softmax(scale * Q K^T) V with heads inside the channel dim (unet:406-416)
+# ----------------------------------------------------------------------------------------------
 def _gemm(A, B, Cm, M, N, K, bo, bi, a, b, c, alpha=1.0, accumulate=False):
     d = _lib.GemmDesc()
     d.M, d.N, d.K, d.batch_outer, d.batch_inner = M, N, K, bo, bi
@@ -1291,9 +1239,7 @@ class _SdpaFn(Function):
         heads, scale_ = ctx.cfg
         B, Lq, Cc = q.shape
         Lk = k.shape[1]
-        dO = dO.contiguous()
-        if dO.dtype != q.dtype:
-            dO = dO.to(q.dtype)
+        dO = _grad_in(dO, q.dtype)
         dQ, dK, dV = torch.empty_like(q), torch.empty_like(k), torch.empty_like(v)
         _sdpa_bwd_unfused(q, k, v, P, dO, dQ, dK, dV, B, Lq, Lk, Cc, heads, scale_, Cc, Cc)
         return dQ, dK, dV, None, None
@@ -1330,17 +1276,12 @@ class _QkvSdpaFn(Function):
     @staticmethod
     def backward(ctx, dO):
         heads, scale_, order, use_flash, (B, L, Cc) = ctx.cfg
-        dO = dO.contiguous()
         C3 = 3 * Cc
         if use_flash:
             qc, kc, vc, O, lse = ctx.saved_tensors
-            if dO.dtype != qc.dtype:
-                dO = dO.to(qc.dtype)
+            dO = _grad_in(dO, qc.dtype)
             dqkv = torch.empty((B, L, C3), dtype=qc.dtype, device=qc.device)
-            dq, dk, dv = torch.empty_like(qc), torch.empty_like(kc), torch.empty_like(vc)
-            delta = torch.empty((B * heads, L), dtype=torch.float32, device=qc.device)
-            call("mig_flash_attention_bwd", _ptr(qc), _ptr(kc), _ptr(vc), _ptr(O), _ptr(dO), _ptr(lse), _ptr(delta), _ptr(dq),
-                 _ptr(dk), _ptr(dv), B, heads, L, L, Cc // heads, float(scale_), _stream())
+            dq, dk, dv = _flash_bwd(qc, kc, vc, O, lse, dO, heads, scale_)
             parts = {"q": dq, "k": dk, "v": dv}
             rows = B * L
             a, b_, c = (parts[n] for n in order)
@@ -1350,8 +1291,7 @@ class _QkvSdpaFn(Function):
             call("mig_concat_channels", _dt(a), _ptr(ab), _ptr(c), _ptr(dqkv), rows, 2 * Cc, Cc, _stream())
             return dqkv, None, None, None
         qkv, P = ctx.saved_tensors
-        if dO.dtype != qkv.dtype:
-            dO = dO.to(qkv.dtype)
+        dO = _grad_in(dO, qkv.dtype)
         dqkv = torch.empty_like(qkv)
         sl = {name: qkv[:, :, i * Cc:(i + 1) * Cc] for i, name in enumerate(order)}
         dsl = {name: dqkv[:, :, i * Cc:(i + 1) * Cc] for i, name in enumerate(order)}
@@ -1441,6 +1381,17 @@ def _flash_fwd(q, k, v, heads: int, scale_: float):
     return out, lse
 
 
+def _flash_bwd(q, k, v, out, lse, dO, heads: int, scale_: float):
+    """Gradients (dq, dk, dv) of _flash_fwd on contiguous q / k / v; dO contiguous in q's dtype."""
+    B, Lq, Cc = q.shape
+    Lk = k.shape[1]
+    dq, dk, dv = torch.empty_like(q), torch.empty_like(k), torch.empty_like(v)
+    delta = torch.empty((B * heads, Lq), dtype=torch.float32, device=q.device)
+    call("mig_flash_attention_bwd", _ptr(q), _ptr(k), _ptr(v), _ptr(out), _ptr(dO), _ptr(lse), _ptr(delta), _ptr(dq),
+         _ptr(dk), _ptr(dv), B, heads, Lq, Lk, Cc // heads, float(scale_), _stream())
+    return dq, dk, dv
+
+
 def flash_attention(q, k, v, heads: int, scale_: float):
     """softmax(scale * q k^T) v without materialising the score matrix (unet:128-135 / 406-416). No autograd."""
     return _flash_fwd(q, k, v, heads, scale_)[0]
@@ -1460,17 +1411,7 @@ class _FlashSdpaFn(Function):
     @staticmethod
     def backward(ctx, dO):
         q, k, v, out, lse = ctx.saved_tensors
-        heads, scale_ = ctx.cfg
-        B, Lq, Cc = q.shape
-        Lk = k.shape[1]
-        dO = dO.contiguous()
-        if dO.dtype != q.dtype:
-            dO = dO.to(q.dtype)
-        dq, dk, dv = torch.empty_like(q), torch.empty_like(k), torch.empty_like(v)
-        delta = torch.empty((B * heads, Lq), dtype=torch.float32, device=q.device)
-        call("mig_flash_attention_bwd", _ptr(q), _ptr(k), _ptr(v), _ptr(out), _ptr(dO), _ptr(lse), _ptr(delta), _ptr(dq),
-             _ptr(dk), _ptr(dv), B, heads, Lq, Lk, Cc // heads, float(scale_), _stream())
-        return dq, dk, dv, None, None
+        return (*_flash_bwd(q, k, v, out, lse, _grad_in(dO, q.dtype), *ctx.cfg), None, None)
 
 
 # ----------------------------------------------------------------------------------------------
@@ -1487,23 +1428,32 @@ def timestep_embedding(timesteps, dim: int, dtype=torch.float32, max_period: int
     return out
 
 
+def _mse_forward(a, b, l1):
+    """mean((a - b)^2), or mean |a - b| when l1, as an fp32 scalar; a and b share shape, dtype and strides."""
+    out = torch.empty((), dtype=torch.float32, device=a.device)
+    partials = torch.empty(2048, dtype=torch.float32, device=a.device)
+    call("mig_mse_fwd", _dt(a), _ptr(a), _ptr(b), _ptr(out), _ptr(partials), a.numel(), int(l1), _stream())
+    return out
+
+
+def _mse_backward(a, b, l1, g):
+    """Gradient w.r.t. a of _mse_forward, given the gradient g of the scalar."""
+    g = g.float().contiguous()
+    da = torch.empty_like(a)
+    call("mig_mse_bwd", _dt(a), _ptr(a), _ptr(b), _ptr(g), _ptr(da), a.numel(), int(l1), _stream())
+    return da
+
+
 class _MseFn(Function):
     @staticmethod
     def forward(ctx, a, b, l1):
-        out = torch.empty((), dtype=torch.float32, device=a.device)
-        partials = torch.empty(2048, dtype=torch.float32, device=a.device)
-        call("mig_mse_fwd", _dt(a), _ptr(a), _ptr(b), _ptr(out), _ptr(partials), a.numel(), int(l1), _stream())
         ctx.save_for_backward(a, b)
         ctx.l1 = l1
-        return out
+        return _mse_forward(a, b, l1)
 
     @staticmethod
     def backward(ctx, g):
-        a, b = ctx.saved_tensors
-        g = g.float().contiguous()
-        da = torch.empty_like(a)
-        call("mig_mse_bwd", _dt(a), _ptr(a), _ptr(b), _ptr(g), _ptr(da), a.numel(), int(ctx.l1), _stream())
-        return da, None, None
+        return _mse_backward(*ctx.saved_tensors, ctx.l1, g), None, None
 
 
 def _pair(a, b):
