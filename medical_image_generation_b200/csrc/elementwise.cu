@@ -1192,9 +1192,10 @@ __global__ void __launch_bounds__(256) adamw_kernel(float* __restrict__ p, const
   }
   float clip = 1.f;
   if (a.max_norm > 0.f && sumsq) {
-    // torch.nn.utils.clip_grad_norm_: coef = max_norm / (total_norm + 1e-6), clamped to 1
+    // torch.nn.utils.clip_grad_norm_: coef = max_norm / (total_norm + 1e-6), clamped to 1. The clamp keeps a NaN
+    // (a NaN anywhere in the gradient): every parameter becomes NaN, as in torch, instead of taking an unclipped step
     float c = a.max_norm / (sqrtf(sumsq[0]) + 1e-6f);
-    clip = c < 1.f ? c : 1.f;
+    clip = (c < 1.f || isnan(c)) ? c : 1.f;
   }
   auto upd = [&](float& pi, float gi, float& mi, float& vi) {
     gi *= clip;

@@ -62,6 +62,48 @@ def assert_close_local(got, want, *, glob, row, col, what) -> dict:
     return errs
 
 
+def f32(x: float) -> float:
+    """`x` rounded to fp32: the value a hyperparameter has after crossing the C ABI as a float."""
+    return float(torch.tensor(x, dtype=torch.float32))
+
+
+def clip_adamw_reference(params, grads, exp_avgs, exp_avg_sqs, step, *, lr, betas, eps, weight_decay, max_norm):
+    """fp64 restatement of torch.nn.utils.clip_grad_norm_(max_norm) followed by ONE torch.optim.AdamW step (decoupled
+    weight decay, bias corrections 1 - beta**step). Every tensor is taken to float64; max_norm 0 / None: no clipping.
+    Returns (params, exp_avgs, exp_avg_sqs, total_norm, clip_coef) after the step (new float64 tensors). As in torch, the
+    clamp of the clip coefficient keeps a NaN: a NaN in any gradient makes every parameter NaN."""
+    d = lambda ts: [t.detach().to(torch.float64) for t in ts]  # noqa: E731
+    ps, gs, ms, vs = d(params), d(grads), d(exp_avgs), d(exp_avg_sqs)
+    total = torch.stack([g.pow(2).sum() for g in gs]).sum().sqrt()
+    coef = torch.ones((), dtype=torch.float64)
+    if max_norm:
+        coef = torch.clamp(max_norm / (total + 1e-6), max=1.0)
+    b1, b2 = betas
+    bc1, bc2 = 1 - b1 ** step, 1 - b2 ** step
+    out_p, out_m, out_v = [], [], []
+    for p, g, m, v in zip(ps, gs, ms, vs):
+        g = g * coef
+        p = p * (1 - lr * weight_decay)
+        m = b1 * m + (1 - b1) * g
+        v = b2 * v + (1 - b2) * g * g
+        p = p - (lr / bc1) * m / (v.sqrt() / bc2 ** 0.5 + eps)
+        out_p.append(p), out_m.append(m), out_v.append(v)
+    return out_p, out_m, out_v, total, coef
+
+
+def adam_step_scale(m_scale, v, step, *, lr, betas, eps):
+    """Magnitude of the Adam step lr / bc1 * m / (sqrt(v) / sqrt(bc2) + eps) with |m| replaced by `m_scale`, the sum of the
+    magnitudes of the terms m is made of: where those terms cancel, the step is small but its rounding error is not."""
+    b1, b2 = betas
+    return lr / (1 - b1 ** step) * m_scale / (v.sqrt() / (1 - b2 ** step) ** 0.5 + eps)
+
+
+def ulp32(x):
+    """Spacing of fp32 numbers at |x| (float64 tensor on x's device)."""
+    a = x.detach().to(torch.float32).abs()
+    return (torch.nextafter(a, torch.full_like(a, float("inf"))) - a).double()
+
+
 def graph_vs_eager(tr_graph, tr_eager, batches):
     """Runs `tr_graph` (cuda_graph=True) and `tr_eager` (same initial state) side by side over `batches`; the eager
     trainer is fed the noise and timesteps the graphed step drew. During capture those tensors are allocated in the
