@@ -315,14 +315,6 @@ __global__ void __launch_bounds__(256) attn_delta_kernel(const __nv_bfloat16* __
   if (lane == 0) delta[(b * H + h) * L + q] = acc;
 }
 
-static int fb_map(CUtensorMap* m, const void* base, int B, int H, int L, int dh, uint32_t box_rows) {
-  const uint64_t C = (uint64_t)H * dh;
-  uint64_t dims[4] = {(uint64_t)dh, (uint64_t)H, (uint64_t)L, (uint64_t)B};
-  uint64_t strides[3] = {(uint64_t)dh * 2, C * 2, (uint64_t)L * C * 2};
-  uint32_t box[4] = {64, 1, box_rows, 1};
-  return make_map(m, base, 4, dims, strides, box);
-}
-
 template <int MODE>
 static int launch_flash_bwd(const CUtensorMap& x1, const CUtensorMap& y1, const CUtensorMap& x2, const CUtensorMap& y2,
                             const CUtensorMap& b1, const CUtensorMap& b2, FlashBwdParams p, dim3 grid, cudaStream_t st) {
@@ -366,9 +358,11 @@ extern "C" int mig_flash_attention_bwd(const void* q, const void* k, const void*
     if (int rc = check_launch("attn_delta_kernel")) return rc;
   }
   CUtensorMap q128, k128, v128, do128, q64, k64, do64;
-  if (fb_map(&q128, q, B, H, Lq, dh, 128) || fb_map(&k128, k, B, H, Lk, dh, 128) || fb_map(&v128, v, B, H, Lk, dh, 128) ||
-      fb_map(&do128, d_o, B, H, Lq, dh, 128) || fb_map(&q64, q, B, H, Lq, dh, 64) || fb_map(&k64, k, B, H, Lk, dh, 64) ||
-      fb_map(&do64, d_o, B, H, Lq, dh, 64))
+  const int64_t ld = (int64_t)H * dh;
+  if (bhld_map(&q128, q, B, H, Lq, dh, 128, ld) || bhld_map(&k128, k, B, H, Lk, dh, 128, ld) ||
+      bhld_map(&v128, v, B, H, Lk, dh, 128, ld) || bhld_map(&do128, d_o, B, H, Lq, dh, 128, ld) ||
+      bhld_map(&q64, q, B, H, Lq, dh, 64, ld) || bhld_map(&k64, k, B, H, Lk, dh, 64, ld) ||
+      bhld_map(&do64, d_o, B, H, Lq, dh, 64, ld))
     return 1;
   FlashBwdParams p{};
   p.B = B; p.H = H; p.Lq = Lq; p.Lk = Lk; p.dh = dh;

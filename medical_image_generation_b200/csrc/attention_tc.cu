@@ -704,15 +704,6 @@ __global__ void __launch_bounds__(FP_THREADS, 1) flash_pair_kernel(const __grid_
   }
 }
 
-// 4-d map over a (B, L, H*dh) bf16 tensor with row pitch ld >= H*dh elements (contiguous: ld = H*dh):
-// dims (dh, H, L, B); box (64, 1, rows, 1)
-static int bhld_map(CUtensorMap* m, const void* base, int B, int H, int L, int dh, uint32_t box_rows, int64_t ld) {
-  uint64_t dims[4] = {(uint64_t)dh, (uint64_t)H, (uint64_t)L, (uint64_t)B};
-  uint64_t strides[3] = {(uint64_t)dh * 2, (uint64_t)ld * 2, (uint64_t)L * (uint64_t)ld * 2};
-  uint32_t box[4] = {64, 1, box_rows, 1};
-  return make_map(m, base, 4, dims, strides, box);
-}
-
 bool flash_eligible(int H, int dh) {
   if (dh % 64 != 0) return false;
   if (dh > 256 && dh % 256 != 0) return false;

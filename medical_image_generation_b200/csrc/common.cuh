@@ -32,6 +32,8 @@ struct DeviceInfo {
 const DeviceInfo& device_info();
 
 inline cudaStream_t as_stream(void* s) { return reinterpret_cast<cudaStream_t>(s); }
+// 16-byte aligned (nullptr counts as aligned)
+inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
 
 // Opt-in to > 48 KB of dynamic shared memory. cudaFuncSetAttribute is PER DEVICE, so the "already done" state is kept per
 // device (one process may drive several GPUs); atomics make concurrent first calls from several host threads benign (the

@@ -64,7 +64,6 @@ static bool tma_enabled() {
   }
   return v == 1;
 }
-static bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
 static int taps(const mig_conv_geom* g) { return g->ksize[0] * g->ksize[1] * g->ksize[2]; }
 static int64_t esize(int dtype) { return dtype == MIG_BF16 ? 2 : 4; }
 static int64_t in_vox(const mig_conv_geom* g) { return (int64_t)g->N * g->in_dims[0] * g->in_dims[1] * g->in_dims[2]; }

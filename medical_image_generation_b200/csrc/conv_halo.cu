@@ -16,6 +16,7 @@
 #include <cuda.h>
 
 #include "common.cuh"
+#include "residue_classes.cuh"
 #include "tc_common.cuh"
 #include "tc_host.cuh"
 
@@ -316,6 +317,15 @@ struct HaloProblem {
   int os[3], oo[3], tgt[3];   // row -> output coordinate = row*os + oo inside tgt[]
 };
 
+// 5-d map (C, W, H, D, N) with box (C, bx, by, bz, 1), no swizzle: staging rows are plain voxels of C channels
+static int halo_map(CUtensorMap* m, const void* base, int N, int D, int H, int W, int C, int bx, int by, int bz) {
+  const uint64_t dims[5] = {(uint64_t)C, (uint64_t)W, (uint64_t)H, (uint64_t)D, (uint64_t)N};
+  const uint64_t strides[4] = {(uint64_t)C * 2, (uint64_t)W * C * 2, (uint64_t)H * W * C * 2,
+                               (uint64_t)D * H * W * C * 2};
+  const uint32_t box[5] = {(uint32_t)C, (uint32_t)bx, (uint32_t)by, (uint32_t)bz, 1};
+  return make_map(m, base, 5, dims, strides, box, "halo map", CU_TENSOR_MAP_SWIZZLE_NONE);
+}
+
 static int launch_halo(const HaloProblem& h, const void* src, const void* wk, const float* bias, const float* chan_bias,
                        const void* residual, void* out, void* stream) {
   HaloParams p{};
@@ -334,19 +344,8 @@ static int launch_halo(const HaloProblem& h, const void* src, const void* wk, co
   p.bias = bias; p.chan_bias = chan_bias;
   p.residual = (const __nv_bfloat16*)residual;
   p.out = (__nv_bfloat16*)out;
-  // 5-d source map (C, W, H, D, N), box (32, hx, hy, hz, 1), no swizzle: staging rows are plain 64-byte voxels
-  EncodeTiledFn enc = get_encode();
-  MIG_REQUIRE(enc != nullptr, "cuTensorMapEncodeTiled unavailable");
   CUtensorMap xm;
-  cuuint64_t gd[5] = {(cuuint64_t)H_C, (cuuint64_t)p.W, (cuuint64_t)p.H, (cuuint64_t)p.D, (cuuint64_t)p.N};
-  cuuint64_t gs[4] = {(cuuint64_t)H_C * 2, (cuuint64_t)p.W * H_C * 2, (cuuint64_t)p.H * p.W * H_C * 2,
-                      (cuuint64_t)p.D * p.H * p.W * H_C * 2};
-  cuuint32_t bx[5] = {(cuuint32_t)H_C, (cuuint32_t)p.hx, (cuuint32_t)p.hy, (cuuint32_t)p.hz, 1};
-  cuuint32_t es[5] = {1, 1, 1, 1, 1};
-  CUresult r = enc(&xm, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5, const_cast<void*>(src), gd, gs, bx, es,
-                   CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  MIG_REQUIRE(r == CUDA_SUCCESS, "cuTensorMapEncodeTiled(halo map) failed with %d", (int)r);
+  if (halo_map(&xm, src, p.N, p.D, p.H, p.W, H_C, p.hx, p.hy, p.hz)) return 1;
   const int T = p.ks[0] * p.ks[1] * p.ks[2];
   const int nvox = p.hz * p.hy * p.hx;
   const int nstg = p.Npad > 32 ? 1 : 2;
@@ -379,23 +378,8 @@ static int run_halo(const mig_conv_geom* g, int which, const void* src, const vo
 // ---------------------------------------------------------------------------------------------------
 // strided dgrad (the backward of the 32-channel Downsample convolution) by stride-residue classes
 // ---------------------------------------------------------------------------------------------------
-// Same decomposition as conv_tma.cu: input voxels with the same residue (i + pad) mod stride see the same tap subset, so
-// every class is a dense stride-1 problem with a sub-filter (8 classes of 1..8 taps for k = 3, s = 2), whose rows
-// scatter into dx with the stride. Here each class runs on the halo kernel.
-int filter_transpose_taps(int dtype, const void* w, void* wt, int Cout, int Tn, int Cin, int ntaps, const int* taps,
-                          void* stream);
-
-struct HaloAxisClass { int o, ext, nu, base, rho; };
-static HaloAxisClass halo_axis_class(int in, int k, int s, int p, int rho) {
-  HaloAxisClass a;
-  a.rho = rho;
-  a.o = ((rho - p) % s + s) % s;                  // first input coordinate of the class
-  a.ext = in > a.o ? (in - a.o + s - 1) / s : 0;  // how many input coordinates it holds
-  a.nu = rho < k ? (k - rho + s - 1) / s : 0;     // taps rho, rho+s, ...
-  a.base = (a.o + p - rho) / s;                   // dy coordinate of (class row 0, tap rho)
-  return a;
-}
-
+// Every class (residue_classes.cuh) is a dense stride-1 problem with a sub-filter (8 classes of 1..8 taps for k = 3,
+// s = 2), whose rows scatter into dx with the stride. Here each class runs on the halo kernel.
 bool halo_dgrad_strided_eligible(const mig_conv_geom* g) {
   if (g->Cout != H_C || g->Cin < 1 || g->Cin > 64) return false;
   bool any = false;
@@ -407,56 +391,28 @@ bool halo_dgrad_strided_eligible(const mig_conv_geom* g) {
   const int64_t vox = (int64_t)g->N * g->in_dims[0] * g->in_dims[1] * g->in_dims[2];
   if (vox < 32768) return false;
   for (int r1 = 0; r1 < g->stride[1]; ++r1)
-    if (halo_axis_class(g->in_dims[1], g->ksize[1], g->stride[1], g->pad[1], r1).ext < HT_Y / 2) return false;
+    if (axis_class(g->in_dims[1], g->ksize[1], g->stride[1], g->pad[1], r1).ext < HT_Y / 2) return false;
   for (int r2 = 0; r2 < g->stride[2]; ++r2)
-    if (halo_axis_class(g->in_dims[2], g->ksize[2], g->stride[2], g->pad[2], r2).ext < HT_X) return false;
+    if (axis_class(g->in_dims[2], g->ksize[2], g->stride[2], g->pad[2], r2).ext < HT_X) return false;
   return true;
 }
 
 int halo_conv_dgrad_strided(const mig_conv_geom* g, const void* dy, const void* w, void* dx, void* ws, int64_t ws_bytes,
                             void* stream) {
-  const int T = g->ksize[0] * g->ksize[1] * g->ksize[2];
-  const int64_t wt_bytes = ((int64_t)g->Cin * T * g->Cout * 2 + 255) / 256 * 256 + 27 * 256;
-  MIG_REQUIRE(ws && ws_bytes >= wt_bytes, "conv_dgrad(halo, strided): workspace too small");
-  bool need_zero = false;
-  for (int pass = 0; pass < 2; ++pass) {
-    uint8_t* wp = (uint8_t*)ws;
-    for (int r0 = 0; r0 < g->stride[0]; ++r0)
-      for (int r1 = 0; r1 < g->stride[1]; ++r1)
-        for (int r2 = 0; r2 < g->stride[2]; ++r2) {
-          HaloAxisClass a[3] = {halo_axis_class(g->in_dims[0], g->ksize[0], g->stride[0], g->pad[0], r0),
-                                halo_axis_class(g->in_dims[1], g->ksize[1], g->stride[1], g->pad[1], r1),
-                                halo_axis_class(g->in_dims[2], g->ksize[2], g->stride[2], g->pad[2], r2)};
-          if (a[0].ext == 0 || a[1].ext == 0 || a[2].ext == 0) continue;
-          const int ntaps = a[0].nu * a[1].nu * a[2].nu;
-          if (pass == 0) { need_zero = need_zero || ntaps == 0; continue; }
-          if (ntaps == 0) continue;
-          int taps[27], nt = 0;
-          for (int u0 = 0; u0 < a[0].nu; ++u0)
-            for (int u1 = 0; u1 < a[1].nu; ++u1)
-              for (int u2 = 0; u2 < a[2].nu; ++u2)
-                taps[nt++] = ((a[0].rho + g->stride[0] * u0) * g->ksize[1] + (a[1].rho + g->stride[1] * u1)) * g->ksize[2] +
-                             (a[2].rho + g->stride[2] * u2);
-          if (filter_transpose_taps(MIG_BF16, w, wp, g->Cout, T, g->Cin, nt, taps, stream)) return 2;
-          HaloProblem h{};
-          h.N = g->N;
-          h.sign = -1;
-          h.Cdst = g->Cin;
-          for (int i = 0; i < 3; ++i) {
-            h.src[i] = g->out_dims[i]; h.ext[i] = a[i].ext; h.tgt[i] = g->in_dims[i];
-            h.ks[i] = a[i].nu; h.lo[i] = a[i].base - (a[i].nu - 1);
-            h.os[i] = g->stride[i]; h.oo[i] = a[i].o;
-          }
-          int rc = launch_halo(h, dy, wp, nullptr, nullptr, nullptr, dx, stream);
-          if (rc) return rc;
-          wp += ((int64_t)g->Cin * nt * g->Cout * 2 + 255) / 256 * 256;
-        }
-    if (pass == 0 && need_zero) {   // some input voxels receive no tap at all (kernel 1 with stride 2)
-      const int64_t n = (int64_t)g->N * g->in_dims[0] * g->in_dims[1] * g->in_dims[2] * g->Cin;
-      cudaMemsetAsync(dx, 0, (size_t)n * 2, as_stream(stream));
+  auto launch_class = [&](const ResidueClass& c, const void* wsub) {
+    HaloProblem h{};
+    h.N = g->N;
+    h.sign = -1;
+    h.Cdst = g->Cin;
+    for (int i = 0; i < 3; ++i) {
+      const AxisClass& a = c.a[i];
+      h.src[i] = g->out_dims[i]; h.ext[i] = a.ext; h.tgt[i] = g->in_dims[i];
+      h.ks[i] = a.nu; h.lo[i] = a.base - (a.nu - 1);
+      h.os[i] = g->stride[i]; h.oo[i] = a.o;
     }
-  }
-  return 0;
+    return launch_halo(h, dy, wsub, nullptr, nullptr, nullptr, dx, stream);
+  };
+  return dgrad_by_residue_classes(g, w, dx, ws, ws_bytes, stream, "conv_dgrad(halo, strided)", launch_class);
 }
 
 // ---------------------------------------------------------------------------------------------------
@@ -650,20 +606,6 @@ bool halo_wgrad_eligible(const mig_conv_geom* g) {
   if ((T + 1) / 2 * 32 > 512) return false;
   const int64_t vox = (int64_t)g->N * g->out_dims[0] * g->out_dims[1] * g->out_dims[2];
   return vox >= 32768 && g->out_dims[2] >= HT_X && g->out_dims[1] >= HT_Y / 2;
-}
-
-static int halo_map(CUtensorMap* m, const void* base, int N, int D, int H, int W, int C, int bx_, int by_, int bz_) {
-  EncodeTiledFn enc = get_encode();
-  MIG_REQUIRE(enc != nullptr, "cuTensorMapEncodeTiled unavailable");
-  cuuint64_t gd[5] = {(cuuint64_t)C, (cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)D, (cuuint64_t)N};
-  cuuint64_t gs[4] = {(cuuint64_t)C * 2, (cuuint64_t)W * C * 2, (cuuint64_t)H * W * C * 2, (cuuint64_t)D * H * W * C * 2};
-  cuuint32_t bx[5] = {(cuuint32_t)C, (cuuint32_t)bx_, (cuuint32_t)by_, (cuuint32_t)bz_, 1};
-  cuuint32_t es[5] = {1, 1, 1, 1, 1};
-  CUresult r = enc(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5, const_cast<void*>(base), gd, gs, bx, es,
-                   CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  MIG_REQUIRE(r == CUDA_SUCCESS, "cuTensorMapEncodeTiled(halo map) failed with %d", (int)r);
-  return 0;
 }
 
 int halo_conv_wgrad(const mig_conv_geom* g, const void* x, const void* dy, float* dw, void* stream) {

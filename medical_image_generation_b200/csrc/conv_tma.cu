@@ -23,6 +23,7 @@
 #include <mutex>
 
 #include "common.cuh"
+#include "residue_classes.cuh"
 #include "tc_common.cuh"
 #include "tc_host.cuh"
 
@@ -811,47 +812,56 @@ bool tma_conv_eligible(const mig_conv_geom* g, int which) {
 static int make_act_map(CUtensorMap* m, const void* base, int N, const int32_t dims[3], int C, int bd, int bh, int bw,
                         const int* estride = nullptr) {
   // 5-d (C, W, H, D, N) with a 64-channel x box window
-  EncodeTiledFn enc = get_encode();
-  MIG_REQUIRE(enc != nullptr, "cuTensorMapEncodeTiled unavailable");
-  cuuint64_t gd[5] = {(cuuint64_t)C, (cuuint64_t)dims[2], (cuuint64_t)dims[1], (cuuint64_t)dims[0], (cuuint64_t)N};
-  cuuint64_t gs[4] = {(cuuint64_t)C * 2, (cuuint64_t)dims[2] * C * 2, (cuuint64_t)dims[1] * dims[2] * C * 2,
-                      (cuuint64_t)dims[0] * dims[1] * dims[2] * C * 2};
+  const uint64_t gd[5] = {(uint64_t)C, (uint64_t)dims[2], (uint64_t)dims[1], (uint64_t)dims[0], (uint64_t)N};
+  const uint64_t gs[4] = {(uint64_t)C * 2, (uint64_t)dims[2] * C * 2, (uint64_t)dims[1] * dims[2] * C * 2,
+                          (uint64_t)dims[0] * dims[1] * dims[2] * C * 2};
   // With an element stride s the box SPANS bw*s tensor elements and delivers every s-th one: bw voxels reach shared
   // memory, exactly the source voxels of bw consecutive outputs of a stride-s convolution.
   const int sd = estride ? estride[0] : 1, sh = estride ? estride[1] : 1, sw = estride ? estride[2] : 1;
-  cuuint32_t bx[5] = {64, (cuuint32_t)(bw * sw), (cuuint32_t)(bh * sh), (cuuint32_t)(bd * sd), 1};
-  cuuint32_t es[5] = {1, (cuuint32_t)sw, (cuuint32_t)sh, (cuuint32_t)sd, 1};
+  const uint32_t bx[5] = {64, (uint32_t)(bw * sw), (uint32_t)(bh * sh), (uint32_t)(bd * sd), 1};
+  const uint32_t es[5] = {1, (uint32_t)sw, (uint32_t)sh, (uint32_t)sd, 1};
   MIG_REQUIRE(bx[1] <= 256 && bx[2] <= 256 && bx[3] <= 256, "conv_tma: strided box exceeds the TMA box limit");
-  CUresult r = enc(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5, const_cast<void*>(base), gd, gs, bx, es,
-                   CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  MIG_REQUIRE(r == CUDA_SUCCESS, "cuTensorMapEncodeTiled(5d activation map) failed with %d", (int)r);
-  return 0;
+  return make_map(m, base, 5, gd, gs, bx, "conv_tma activation map", CU_TENSOR_MAP_SWIZZLE_128B, es);
 }
 
-static BoxGeom make_box_geom(const mig_conv_geom* g, int which) {
-  BoxGeom b{};
-  const int32_t* rows = which == 1 ? g->in_dims : g->out_dims;
-  b.N = g->N; b.D = rows[0]; b.H = rows[1]; b.W = rows[2];
+enum BoxPicker { kBox64, kBoxRows, kBoxStage };   // pick_box, pick_box_rows (fwd / dgrad), pick_box_k (wgrad)
+
+// One box-conv problem: rows over ext[] (N samples), source coordinate = row*ss + tap*sign + off over ks[] taps, and
+// row j lands at j*os + oo inside out[]. Returns whether the picker found a box worth using.
+static bool box_geom(BoxGeom& b, BoxPicker pick, int N, const int ext[3], const int ks[3], const int off[3], int sign,
+                     const int ss[3], const int os[3], const int oo[3], const int out[3], int Csrc, int Cdst) {
+  b = BoxGeom{};
+  b.N = N; b.D = ext[0]; b.H = ext[1]; b.W = ext[2];
   b.rb = 64;
-  if (which == 2) pick_box_k(b.D, b.H, b.W, &b.bd, &b.bh, &b.bw);
-  else pick_box_rows(b.D, b.H, b.W, &b.bd, &b.bh, &b.bw, &b.rb);
+  const bool ok = pick == kBoxRows    ? pick_box_rows(b.D, b.H, b.W, &b.bd, &b.bh, &b.bw, &b.rb)
+                  : pick == kBoxStage ? pick_box_k(b.D, b.H, b.W, &b.bd, &b.bh, &b.bw)
+                                      : pick_box(b.D, b.H, b.W, &b.bd, &b.bh, &b.bw);
   b.nb = b.bd * b.bh * b.bw;
   set_box_counts(b);
   int taps = 1;
   for (int i = 0; i < 3; ++i) {
-    b.ks[i] = g->ksize[i];
-    b.off[i] = which == 1 ? g->pad[i] : -g->pad[i];
-    taps *= g->ksize[i];
+    b.ks[i] = ks[i]; b.off[i] = off[i]; b.ss[i] = ss[i]; b.os[i] = os[i]; b.oo[i] = oo[i];
+    taps *= ks[i];
   }
-  b.sign = which == 1 ? -1 : 1;
-  for (int i = 0; i < 3; ++i) b.ss[i] = which == 1 ? 1 : g->stride[i];
-  b.Csrc = which == 1 ? g->Cout : g->Cin;
-  b.Cdst = which == 1 ? g->Cin : g->Cout;
-  b.K = taps * b.Csrc;
-  b.cchunks = (b.Csrc + 63) / 64;
-  for (int i = 0; i < 3; ++i) { b.os[i] = 1; b.oo[i] = 0; }
-  b.OD = b.D; b.OH = b.H; b.OW = b.W;
+  b.sign = sign;
+  b.Csrc = Csrc; b.Cdst = Cdst;
+  b.K = taps * Csrc;
+  b.cchunks = (Csrc + 63) / 64;
+  b.OD = out[0]; b.OH = out[1]; b.OW = out[2];
+  return ok;
+}
+
+static const int kOnes[3] = {1, 1, 1}, kZeros[3] = {0, 0, 0};
+
+// which: 0 fwd, 1 dgrad, 2 wgrad of a convolution; rows are the tensor being produced (wgrad: the conv output)
+static BoxGeom make_box_geom(const mig_conv_geom* g, int which) {
+  const int32_t* rows = which == 1 ? g->in_dims : g->out_dims;
+  int off[3];
+  for (int i = 0; i < 3; ++i) off[i] = which == 1 ? g->pad[i] : -g->pad[i];
+  BoxGeom b;
+  box_geom(b, which == 2 ? kBoxStage : kBoxRows, g->N, rows, g->ksize, off, which == 1 ? -1 : 1,
+           which == 1 ? kOnes : g->stride, kOnes, kZeros, rows, which == 1 ? g->Cout : g->Cin,
+           which == 1 ? g->Cin : g->Cout);
   return b;
 }
 
@@ -883,13 +893,24 @@ static int launch_box_conv(const BoxGeom& b, int N, const int32_t* sdims, const 
 // fill time (ncu: the L2 -> SM path sustains ~60-85 B/clk/SM); a CTA adds a fixed launch / pipeline-fill / drain cost
 // (ncu on 64-channel layers: ~15 k cycles around a 3.5 k-cycle main loop, which is why narrow layers also get
 // 256-row tiles); the grid runs in ceil(CTAs / SMs) waves; split-K fills the chip on the small deep levels.
-static void plan_box_conv(const BoxGeom& b, int bn, int num_kb, bool ws_ok, int* mt, int* splits) {
+// Split-K needs an fp32 [M][Cdst] workspace: ws_bytes is what the launch has (0: none, as for the class launches).
+struct BoxPlan {
+  int bn, mt;              // output-channel tile, stacked 128-row accumulators
+  int num_kb;              // k-blocks: taps x 64-channel chunks
+  int splits, kb_per_split;
+};
+static BoxPlan plan_box(const BoxGeom& b, int64_t ws_bytes) {
   const int sms = device_info().sm_count;
+  BoxPlan pl;
+  pl.bn = pick_bn(b.Cdst);
+  pl.num_kb = (b.K / b.Csrc) * b.cchunks;
+  const int bn = pl.bn, num_kb = pl.num_kb;
   const int64_t ntiles = (b.Cdst + bn - 1) / bn;
   const int64_t M = (int64_t)b.N * b.D * b.H * b.W;
+  const bool ws_ok = ws_bytes >= M * b.Cdst * 4;
   double best = 1e30;
   static const int cand_s[] = {1, 2, 3, 4, 6, 8, 12, 16};
-  *mt = 1; *splits = 1;
+  pl.mt = 1; pl.splits = 1;
   for (int m_ = 1; m_ <= 2; ++m_) {
     const int nslot_ = m_ * (TBM / b.rb);
     const int64_t mtiles_ = (b.num_boxes + nslot_ - 1) / nslot_;
@@ -901,9 +922,12 @@ static void plan_box_conv(const BoxGeom& b, int bn, int num_kb, bool ws_ok, int*
       const double t_epi = 2500.0 + m_ * (bn / 16) * (s_ > 1 ? 160.0 : 110.0);
       double t = waves * (kb * t_stage + t_epi + 9000.0);
       if (s_ > 1) t += (double)M * b.Cdst * 14.0 / 3000.0 + 8000.0;   // memset + fp32 reductions + finish pass
-      if (t < best) { best = t; *mt = m_; *splits = s_; }
+      if (t < best) { best = t; pl.mt = m_; pl.splits = s_; }
     }
   }
+  pl.kb_per_split = (num_kb + pl.splits - 1) / pl.splits;
+  pl.splits = (num_kb + pl.kb_per_split - 1) / pl.kb_per_split;
+  return pl;
 }
 
 // One TileCounter per launch out of a per-device pool, handed out round-robin: launches in flight (and the kernel nodes
@@ -951,13 +975,14 @@ static TileCounter* next_tile_counter(cudaStream_t st) {
 // tile i overlaps the main loop of tile i+1. For the 256 x 256 tile the epilogue is exposed, and measured on the
 // config-3 step the extra reduction work cost 0.8 ms of convolution time per step to save 0.16 ms of (L2-resident)
 // statistics passes -- there the separate pass is the faster design. MIG_GN_EPILOGUE=always / never overrides (tests).
-static bool epilogue_stats_ok(const BoxGeom& b, int bn, int mt, int splits, int groups) {
-  if (!(splits == 1 && bn >= 64 && b.Cdst % 16 == 0 && groups > 0 && b.Cdst % groups == 0 && (b.Cdst / groups) % 8 == 0))
+static bool epilogue_stats_ok(const BoxGeom& b, const BoxPlan& pl, int groups) {
+  if (!(pl.splits == 1 && pl.bn >= 64 && b.Cdst % 16 == 0 && groups > 0 && b.Cdst % groups == 0 &&
+        (b.Cdst / groups) % 8 == 0))
     return false;
   const char* e = getenv("MIG_GN_EPILOGUE");
   if (e && e[0] == 'a') return true;
   if (e && e[0] == 'n') return false;
-  return 2 * mt * bn <= 512;
+  return 2 * pl.mt * pl.bn <= 512;
 }
 
 // src: activation being convolved (x for fwd, dy for dgrad); wk: filter as [Cdst][taps][Csrc] (or, with ex->bmn, as
@@ -977,7 +1002,8 @@ static int launch_box_conv(const BoxGeom& b, int N, const int32_t* sdims, const 
   cudaStream_t st = as_stream(stream);
   CUtensorMap xm, wm;
   if (make_act_map(&xm, src, N, sdims, b.Csrc, b.bd, b.bh, b.bw, b.ss)) return 1;
-  const int bn = b.Cdst > 128 ? 256 : (b.Cdst > 64 ? 128 : (b.Cdst > 32 ? 64 : 32));
+  const BoxPlan pl = plan_box(b, ws ? ws_bytes : 0);
+  const int bn = pl.bn, mt = pl.mt, splits = pl.splits;
   const bool bmn = ex && ex->bmn;
   if (bmn) {
     MIG_REQUIRE(bn >= 64, "conv_tma: the MN-major filter operand needs at least 64 output channels");
@@ -997,21 +1023,18 @@ static int launch_box_conv(const BoxGeom& b, int N, const int32_t* sdims, const 
   p.bias = bias; p.chan_bias = chan_bias;
   p.residual = (const __nv_bfloat16*)residual;
   p.out = (__nv_bfloat16*)out;
-  p.num_kb = (b.K / b.Csrc) * b.cchunks;   // taps x channel chunks
+  p.num_kb = pl.num_kb;
+  p.kb_per_split = pl.kb_per_split;
   const int sms = device_info().sm_count;
   const int64_t ntiles = (b.Cdst + bn - 1) / bn;
   const int64_t M = (int64_t)b.N * b.D * b.H * b.W;
-  int mt = 1, splits = 1;
-  plan_box_conv(b, bn, p.num_kb, ws != nullptr && ws_bytes >= M * b.Cdst * 4, &mt, &splits);
   const int nslot = mt * (TBM / b.rb);
   const int64_t mtiles = (b.num_boxes + nslot - 1) / nslot;
-  p.kb_per_split = (p.num_kb + splits - 1) / splits;
-  splits = (p.num_kb + p.kb_per_split - 1) / p.kb_per_split;
   if (splits > 1) {
     p.partial = (float*)ws;
     cudaMemsetAsync(ws, 0, (size_t)(M * b.Cdst * 4), st);
   }
-  if (ex && ex->gn_sums && epilogue_stats_ok(b, bn, mt, splits, ex->gn_groups)) {
+  if (ex && ex->gn_sums && epilogue_stats_ok(b, pl, ex->gn_groups)) {
     p.gn_sums = ex->gn_sums;
     p.gn_G = ex->gn_groups;
     p.gn_cpg = b.Cdst / ex->gn_groups;
@@ -1055,8 +1078,8 @@ static int launch_box_conv(const BoxGeom& b, int N, const int32_t* sdims, const 
   else rc = launch_conv_tma<32, 1>(xm, wm, p, grid, st);
   if (rc) return rc;
   if (splits > 1) {
-    auto al16 = [](const void* q) { return (reinterpret_cast<uintptr_t>(q) & 15) == 0; };
-    if (b.Cdst % 8 == 0 && al16(ws) && al16(bias) && al16(chan_bias) && al16(residual) && al16(out))
+    if (b.Cdst % 8 == 0 && aligned16(ws) && aligned16(bias) && aligned16(chan_bias) && aligned16(residual) &&
+        aligned16(out))
       tma_splitk_finish8<<<bw_grid(M * b.Cdst / 8, 256), 256, 0, st>>>((const float*)ws, bias, chan_bias,
                                                                        (const __nv_bfloat16*)residual,
                                                                        (__nv_bfloat16*)out, M, b.Cdst,
@@ -1085,15 +1108,8 @@ int tma_conv_fwd(const mig_conv_geom* g, const void* x, const void* w, const flo
 
 // would tma_conv_fwd's epilogue produce the GroupNorm statistics for this geometry / workspace?
 bool tma_conv_fwd_stats_in_epilogue(const mig_conv_geom* g, int gn_groups, int64_t ws_bytes) {
-  BoxGeom b = make_box_geom(g, 0);
-  const int bn = b.Cdst > 128 ? 256 : (b.Cdst > 64 ? 128 : (b.Cdst > 32 ? 64 : 32));
-  const int num_kb = (b.K / b.Csrc) * b.cchunks;
-  const int64_t M = (int64_t)b.N * b.D * b.H * b.W;
-  int mt, splits;
-  plan_box_conv(b, bn, num_kb, ws_bytes >= M * b.Cdst * 4, &mt, &splits);
-  const int kbs = (num_kb + splits - 1) / splits;
-  splits = (num_kb + kbs - 1) / kbs;
-  return epilogue_stats_ok(b, bn, mt, splits, gn_groups);
+  const BoxGeom b = make_box_geom(g, 0);
+  return epilogue_stats_ok(b, plan_box(b, ws_bytes), gn_groups);
 }
 
 int tma_conv_dgrad(const mig_conv_geom* g, const void* dy, const void* w, void* dx, void* ws, int64_t ws_bytes,
@@ -1119,24 +1135,7 @@ int tma_conv_dgrad(const mig_conv_geom* g, const void* dy, const void* w, void* 
 // ---------------------------------------------------------------------------------------------------
 // strided dgrad by stride-residue classes
 // ---------------------------------------------------------------------------------------------------
-// dx[i] = sum_t dy[(i + p - t)/s] w[t] over the taps with (i + p - t) % s == 0. Input voxels with the same residue
-// rho = (i + p) mod s (per axis) see the same tap subset {rho, rho+s, ...}; writing i = s*j + o and t = rho + s*u
-// gives dx_class[j] = sum_u dy[j - u + base] w[rho + s*u]: a dense stride-1 problem per class (2^d classes for
-// stride 2), whose rows scatter back to dx with stride s. Total work = the useful work (no zero taps).
-int filter_transpose_taps(int dtype, const void* w, void* wt, int Cout, int Tn, int Cin, int ntaps, const int* taps,
-                          void* stream);
-
-struct AxisClass { int o, ext, nu, base, rho; };
-static AxisClass axis_class(int in, int k, int s, int p, int rho) {
-  AxisClass a;
-  a.rho = rho;
-  a.o = ((rho - p) % s + s) % s;
-  a.ext = in > a.o ? (in - a.o + s - 1) / s : 0;
-  a.nu = rho < k ? (k - rho + s - 1) / s : 0;
-  a.base = (a.o + p - rho) / s;
-  return a;
-}
-
+// Every class (residue_classes.cuh) runs as a dense stride-1 box problem on the conv kernel, without split-K.
 bool tma_dgrad_strided_eligible(const mig_conv_geom* g) {
   bool any = false;
   for (int i = 0; i < 3; ++i) {
@@ -1144,79 +1143,26 @@ bool tma_dgrad_strided_eligible(const mig_conv_geom* g) {
     any = any || g->stride[i] == 2;
   }
   if (!any || g->Cout % 64 != 0 || g->Cin < 8) return false;
-  for (int r0 = 0; r0 < g->stride[0]; ++r0)
-    for (int r1 = 0; r1 < g->stride[1]; ++r1)
-      for (int r2 = 0; r2 < g->stride[2]; ++r2) {
-        AxisClass a[3] = {axis_class(g->in_dims[0], g->ksize[0], g->stride[0], g->pad[0], r0),
-                          axis_class(g->in_dims[1], g->ksize[1], g->stride[1], g->pad[1], r1),
-                          axis_class(g->in_dims[2], g->ksize[2], g->stride[2], g->pad[2], r2)};
-        if (a[0].ext == 0 || a[1].ext == 0 || a[2].ext == 0) continue;
-        if (a[0].nu * a[1].nu * a[2].nu > 32) return false;
-        int bd, bh, bw;
-        if (!pick_box(a[0].ext, a[1].ext, a[2].ext, &bd, &bh, &bw)) return false;
-      }
+  ResidueClass cls[kMaxClasses];
+  const int n = residue_classes(g, cls);
+  for (int i = 0; i < n; ++i) {
+    const AxisClass* a = cls[i].a;
+    int bd, bh, bw;
+    if (cls[i].ntaps > kMaxClassTaps || !pick_box(a[0].ext, a[1].ext, a[2].ext, &bd, &bh, &bw)) return false;
+  }
   return true;
 }
 
 int tma_conv_dgrad_strided(const mig_conv_geom* g, const void* dy, const void* w, void* dx, void* ws, int64_t ws_bytes,
                            void* stream) {
-  const int T = g->ksize[0] * g->ksize[1] * g->ksize[2];
-  const int64_t wt_bytes = ((int64_t)g->Cin * T * g->Cout * 2 + 255) / 256 * 256 + 27 * 256;
-  MIG_REQUIRE(ws && ws_bytes >= wt_bytes, "conv_dgrad(tma, strided): workspace too small");
-  cudaStream_t st = as_stream(stream);
-  bool need_zero = false;
-  uint8_t* wp = (uint8_t*)ws;
-  for (int r0 = 0; r0 < g->stride[0]; ++r0)
-    for (int r1 = 0; r1 < g->stride[1]; ++r1)
-      for (int r2 = 0; r2 < g->stride[2]; ++r2) {
-        AxisClass a[3] = {axis_class(g->in_dims[0], g->ksize[0], g->stride[0], g->pad[0], r0),
-                          axis_class(g->in_dims[1], g->ksize[1], g->stride[1], g->pad[1], r1),
-                          axis_class(g->in_dims[2], g->ksize[2], g->stride[2], g->pad[2], r2)};
-        if (a[0].ext == 0 || a[1].ext == 0 || a[2].ext == 0) continue;
-        if (a[0].nu * a[1].nu * a[2].nu == 0) need_zero = true;
-      }
-  if (need_zero) {   // some input voxels receive no tap at all (e.g. kernel 1 with stride 2)
-    const int64_t n = (int64_t)g->N * g->in_dims[0] * g->in_dims[1] * g->in_dims[2] * g->Cin;
-    cudaMemsetAsync(dx, 0, (size_t)n * 2, st);
-  }
-  for (int r0 = 0; r0 < g->stride[0]; ++r0)
-    for (int r1 = 0; r1 < g->stride[1]; ++r1)
-      for (int r2 = 0; r2 < g->stride[2]; ++r2) {
-        AxisClass a[3] = {axis_class(g->in_dims[0], g->ksize[0], g->stride[0], g->pad[0], r0),
-                          axis_class(g->in_dims[1], g->ksize[1], g->stride[1], g->pad[1], r1),
-                          axis_class(g->in_dims[2], g->ksize[2], g->stride[2], g->pad[2], r2)};
-        const int ntaps = a[0].nu * a[1].nu * a[2].nu;
-        if (a[0].ext == 0 || a[1].ext == 0 || a[2].ext == 0 || ntaps == 0) continue;
-        int taps[32], nt = 0;
-        for (int u0 = 0; u0 < a[0].nu; ++u0)
-          for (int u1 = 0; u1 < a[1].nu; ++u1)
-            for (int u2 = 0; u2 < a[2].nu; ++u2)
-              taps[nt++] = ((a[0].rho + g->stride[0] * u0) * g->ksize[1] + (a[1].rho + g->stride[1] * u1)) * g->ksize[2] +
-                           (a[2].rho + g->stride[2] * u2);
-        if (filter_transpose_taps(MIG_BF16, w, wp, g->Cout, T, g->Cin, nt, taps, stream)) return 2;
-        BoxGeom b{};
-        b.N = g->N; b.D = a[0].ext; b.H = a[1].ext; b.W = a[2].ext;
-        b.rb = 64;
-        pick_box(b.D, b.H, b.W, &b.bd, &b.bh, &b.bw);
-        b.nb = b.bd * b.bh * b.bw;
-        set_box_counts(b);
-        for (int i = 0; i < 3; ++i) {
-          b.ks[i] = a[i].nu;
-          b.off[i] = a[i].base;
-          b.os[i] = g->stride[i];
-          b.oo[i] = a[i].o;
-        }
-        b.sign = -1;
-        for (int i = 0; i < 3; ++i) b.ss[i] = 1;
-        b.Csrc = g->Cout; b.Cdst = g->Cin;
-        b.K = nt * b.Csrc;
-        b.cchunks = (b.Csrc + 63) / 64;
-        b.OD = g->in_dims[0]; b.OH = g->in_dims[1]; b.OW = g->in_dims[2];
-        int rc = launch_box_conv(b, g->N, g->out_dims, dy, wp, nullptr, nullptr, nullptr, dx, nullptr, 0, stream);
-        if (rc) return rc;
-        wp += ((int64_t)g->Cin * nt * g->Cout * 2 + 255) / 256 * 256;
-      }
-  return 0;
+  auto launch_class = [&](const ResidueClass& c, const void* wsub) {
+    int ext[3], nu[3], base[3], o[3];
+    for (int i = 0; i < 3; ++i) { ext[i] = c.a[i].ext; nu[i] = c.a[i].nu; base[i] = c.a[i].base; o[i] = c.a[i].o; }
+    BoxGeom b;
+    box_geom(b, kBox64, g->N, ext, nu, base, -1, kOnes, g->stride, o, g->in_dims, g->Cout, g->Cin);
+    return launch_box_conv(b, g->N, g->out_dims, dy, wsub, nullptr, nullptr, nullptr, dx, nullptr, 0, stream);
+  };
+  return dgrad_by_residue_classes(g, w, dx, ws, ws_bytes, stream, "conv_dgrad(tma, strided)", launch_class);
 }
 
 // ---------------------------------------------------------------------------------------------------
@@ -1234,26 +1180,10 @@ bool tma_upconv_class_eligible(int N, const int32_t low[3], int Cin, int Cout) {
 int tma_upconv_class_fwd(int N, const int32_t low[3], const int32_t factor[3], const int32_t res[3], const int32_t nu[3],
                          const int32_t base[3], int Cin, int Cout, const void* x, const void* wc, const float* bias,
                          void* y, void* stream) {
-  BoxGeom b{};
-  b.N = N; b.D = low[0]; b.H = low[1]; b.W = low[2];
-  b.rb = 64;
-  MIG_REQUIRE(pick_box(b.D, b.H, b.W, &b.bd, &b.bh, &b.bw), "upconv_fwd: no TMA box for this volume");
-  b.nb = b.bd * b.bh * b.bw;
-  set_box_counts(b);
-  int taps = 1;
-  for (int i = 0; i < 3; ++i) {
-    b.ks[i] = nu[i];
-    b.off[i] = base[i];
-    b.ss[i] = 1;
-    b.os[i] = factor[i];
-    b.oo[i] = res[i];
-    taps *= nu[i];
-  }
-  b.sign = 1;
-  b.Csrc = Cin; b.Cdst = Cout;
-  b.K = taps * Cin;
-  b.cchunks = (Cin + 63) / 64;
-  b.OD = low[0] * factor[0]; b.OH = low[1] * factor[1]; b.OW = low[2] * factor[2];
+  const int out[3] = {low[0] * factor[0], low[1] * factor[1], low[2] * factor[2]};
+  BoxGeom b;
+  MIG_REQUIRE(box_geom(b, kBox64, N, low, nu, base, 1, kOnes, factor, res, out, Cin, Cout),
+              "upconv_fwd: no TMA box for this volume");
   return launch_box_conv(b, N, low, x, wc, bias, nullptr, nullptr, y, nullptr, 0, stream);
 }
 

@@ -7,8 +7,6 @@
 
 namespace mig {
 
-static inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
-
 // ------------------------------------------------------------------------------------------------
 // generic unary / binary maps
 // ------------------------------------------------------------------------------------------------

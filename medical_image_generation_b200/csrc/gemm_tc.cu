@@ -274,8 +274,6 @@ __global__ void __launch_bounds__(256) splitk_finish_kernel(const float* __restr
 // ---------------------------------------------------------------------------------------------------
 // host: tensor maps
 // ---------------------------------------------------------------------------------------------------
-static int pick_bn(int cdst) { return cdst > 128 ? 256 : (cdst > 64 ? 128 : (cdst > 32 ? 64 : 32)); }
-
 template <int BN>
 static int launch_conv_tc(const CUtensorMap& wmap, const ConvTcParams& p, dim3 grid, cudaStream_t st) {
   constexpr int smem = stages_for(BN) * (TBM * 128 + BN * 128) + 1024;

@@ -71,18 +71,10 @@ static GtGeom gt_geom(int N, int64_t S, int C, int G) {
 }
 
 static int gt_map(CUtensorMap* m, const void* base, const GtGeom& g) {
-  EncodeTiledFn enc = get_encode();
-  MIG_REQUIRE(enc != nullptr, "cuTensorMapEncodeTiled unavailable (driver too old?)");
-  cuuint64_t gd[2] = {(cuuint64_t)g.C, (cuuint64_t)((int64_t)g.N * g.S)};
-  cuuint64_t gs[1] = {(cuuint64_t)g.C * 2};
-  cuuint32_t bx[2] = {(cuuint32_t)g.cb, (cuuint32_t)g.R};
-  cuuint32_t es[2] = {1, 1};
-  CUresult r = enc(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(base), gd, gs, bx, es,
-                   CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  MIG_REQUIRE(r == CUDA_SUCCESS, "groupnorm: cuTensorMapEncodeTiled failed with %d (C=%d rows=%lld)", (int)r, g.C,
-              (long long)((int64_t)g.N * g.S));
-  return 0;
+  const uint64_t dims[2] = {(uint64_t)g.C, (uint64_t)((int64_t)g.N * g.S)};
+  const uint64_t strides[1] = {(uint64_t)g.C * 2};
+  const uint32_t box[2] = {(uint32_t)g.cb, (uint32_t)g.R};
+  return make_map(m, base, 2, dims, strides, box, "groupnorm map", CU_TENSOR_MAP_SWIZZLE_NONE);
 }
 
 __device__ __forceinline__ uint4 lds16(uint32_t addr) {

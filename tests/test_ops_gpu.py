@@ -79,6 +79,7 @@ CONV_CASES = [
     (1, 32, 32, (33, 35, 37), (3, 3, 3), (2, 2, 2), (1, 1, 1)),   # odd extents: classes of different size
     (2, 32, 32, (8, 64, 64), (3, 3, 1), (2, 2, 1), (1, 1, 0)),    # anisotropic stride / kernel
     (8, 24, 32, (64, 64), (3, 3), (2, 2), (1, 1)),                # 2-D, 24 input channels
+    (1, 32, 32, (32, 32, 32), (1, 1, 1), (2, 2, 2), (0, 0, 0)),   # kernel 1 stride 2: most input voxels get zero gradient
 ]
 
 
