@@ -335,6 +335,20 @@ int mig_upconv_unfold_wgrad(const float* dwc, float* dw, int32_t Cout, int32_t C
 int mig_class_interleave(int dtype, const void* src, void* dst, int32_t N, const int32_t low[3], const int32_t factor[3],
                          int32_t C, int to_classes, void* stream);
 
+/* ---- SSIM / MS-SSIM validation metrics (ldm:241-330: generative.metrics.SSIMMetric / MultiScaleSSIMMetric) --------
+ * Replaces monai-generative's compute_ssim_and_cs (five depthwise conv{2,3}d with the dense window, then the SSIM and
+ * contrast-structure maps) for a list of image pairs, with the window applied separably and nothing but the inputs in
+ * HBM. a: [na][D][H][W][C], b: [nb][D][H][W][C] (channels-last, same dtype; 2-D images use D = 1, ksize[0] = 1).
+ * pairs: DEVICE int32 [P][2] of (index into a, index into b); a pair with an index out of range gets NaN.
+ * taps_host: the three 1-D windows, D taps then H taps then W taps (ksize[0] + ksize[1] + ksize[2] floats), 1 <= k <= 16
+ * and k <= the extent per axis. "Valid" correlation (extent - k + 1 per axis), c1 = (k1 L)^2, c2 = (k2 L)^2 as given.
+ * out: DEVICE fp64 [P][2] = (mean ssim, mean cs) over channels and valid voxels. Deterministic (fixed-order fp64
+ * reduction, no atomics); workspace = mig_ssim_workspace_bytes(P, C, dims, ksize) (-1: invalid shape). */
+int64_t mig_ssim_workspace_bytes(int32_t P, int32_t C, const int32_t dims[3], const int32_t ksize[3]);
+int mig_ssim_pairs(int dtype, const void* a, const void* b, int32_t na, int32_t nb, const int32_t* pairs, int32_t P,
+                   const int32_t dims[3], int32_t C, const int32_t ksize[3], const float* taps_host, float c1, float c2,
+                   double* out, void* workspace, int64_t workspace_bytes, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

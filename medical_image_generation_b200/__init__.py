@@ -8,8 +8,9 @@ a CUDA device, and raises otherwise.
 """
 from .autoencoderkl import AutoencoderKL
 from .inferers import DiffusionInferer, LatentDiffusionInferer
+from .metrics import MultiScaleSSIMMetric, SSIMMetric, pairwise_ms_ssim
 from .schedulers import DDIMScheduler, DDPMScheduler
 from .unet import DiffusionModelUNet
 
 __all__ = ["AutoencoderKL", "DiffusionModelUNet", "DDPMScheduler", "DDIMScheduler", "DiffusionInferer",
-           "LatentDiffusionInferer"]
+           "LatentDiffusionInferer", "SSIMMetric", "MultiScaleSSIMMetric", "pairwise_ms_ssim"]

@@ -106,10 +106,12 @@ _SIGNATURES = {
     "mig_upconv_fwd": [_p, _p, _p, _p, _i, _I3, _i, _i, _I3, _I3, _I3, _p],
     "mig_upconv_unfold_wgrad": [_p, _p, _i, _i, _I3, _I3, _I3, _p],
     "mig_class_interleave": [_i, _p, _p, _i, _I3, _I3, _i, _i, _p],
+    "mig_ssim_workspace_bytes": [_i, _i, _I3, _I3],
+    "mig_ssim_pairs": [_i, _p, _p, _i, _i, _p, _i, _I3, _i, _I3, _p, _f, _f, _p, _p, _l, _p],
 }
 _RESTYPES = {"mig_last_error": C.c_char_p, "mig_conv_workspace_bytes": C.c_int64,
              "mig_groupnorm_workspace_bytes": C.c_int64, "mig_patch_stats_workspace_bytes": C.c_int64,
-             "mig_upconv_folded_elems": C.c_int64}
+             "mig_upconv_folded_elems": C.c_int64, "mig_ssim_workspace_bytes": C.c_int64}
 
 _lib = None
 

@@ -14,7 +14,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OBJ = os.path.join(HERE, "build")
 LIB = os.path.join(HERE, "libmedimgen_b200.so")
-SOURCES = ["runtime.cu", "elementwise.cu", "groupnorm.cu", "groupnorm_tma.cu", "gemm_simt.cu", "gemm_tc.cu", "gemm_tc2.cu", "conv_tma.cu", "small_ops.cu", "attention_tc.cu", "attention_bwd_tc.cu", "conv_halo.cu", "conv_thin.cu", "conv.cu", "data_path.cu", "upconv.cu"]
+SOURCES = ["runtime.cu", "elementwise.cu", "groupnorm.cu", "groupnorm_tma.cu", "gemm_simt.cu", "gemm_tc.cu", "gemm_tc2.cu", "conv_tma.cu", "small_ops.cu", "attention_tc.cu", "attention_bwd_tc.cu", "conv_halo.cu", "conv_thin.cu", "conv.cu", "data_path.cu", "upconv.cu", "ssim.cu"]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-std=c++17", "-lineinfo", "-Xcompiler", "-fPIC",
          "--expt-relaxed-constexpr", "-Xptxas", "-v"]
