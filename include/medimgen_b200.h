@@ -227,6 +227,20 @@ int mig_ddpm_step(int dtype, const void* model_out, const void* x, const void* z
 int mig_ddim_step(int dtype, const void* model_out, const void* x, const void* z, void* prev, void* x0_hat,
                   int64_t n, float sqrt_acp_t, float sqrt_one_minus_acp_t, float sqrt_acp_prev, float dir_coef,
                   float sigma, int prediction, int clip, void* stream);
+/* one timestep of the DDPM variational bound (monai-generative DiffusionInferer.get_likelihood): per element, from the
+ * model output, the noisy sample x_t and the clean input x0, the KL between the posterior q(x_{t-1} | x_t, x0) and the
+ * model's p(x_{t-1} | x_t) when t > 0, and at t == 0 the negative log-likelihood of x0 under the discretised Gaussian
+ * decoder (bins of 2 * half_bin, tanh approximation of the normal CDF). t = timesteps[b] (device int64 [B]); every
+ * scalar comes from `table`, a device fp32 [T][7] array (table_len == 7 * T): sqrt(acp_t), sqrt(1 - acp_t), c0, ct,
+ * -1 + lv - lv + exp(lv - lv), exp(-lv), exp(-0.5 lv) with lv the log of the scheduler's variance. Writes the fp32 map
+ * in x's element order when kl_map is non-NULL, and ADDS each sample's mean into total (DEVICE fp64 [B]).
+ * prediction: 0 epsilon, 1 sample, 2 v_prediction. Deterministic (fixed-order fp64 reduction, no atomics);
+ * workspace = mig_ddpm_vlb_workspace_bytes(B, per_sample) (-1: invalid shape). */
+int64_t mig_ddpm_vlb_workspace_bytes(int32_t B, int64_t per_sample);
+int mig_ddpm_vlb_term(int dtype, const void* model_out, const void* x_t, const void* x0, const int64_t* timesteps,
+                      const float* table, int64_t table_len, int32_t T, int32_t B, int64_t per_sample, int prediction,
+                      int clip, float half_bin, float* kl_map, double* total, void* workspace, int64_t workspace_bytes,
+                      void* stream);
 
 /* ---- K16/K17: losses --------------------------------------------------------------------------- */
 /* out[0] = mean((a-b)^2) (ldm:169) or mean(|a-b|) (aetrain:414); `partials` needs 2048 floats */

@@ -86,6 +86,8 @@ _SIGNATURES = {
     "mig_ddpm_add_noise": [_i, _p, _p, _p, _p, _p, _i, _l, _i, _i, _p],
     "mig_ddpm_step": [_i, _p, _p, _p, _p, _p, _l, _f, _f, _f, _f, _f, _i, _i, _p],
     "mig_ddim_step": [_i, _p, _p, _p, _p, _p, _l, _f, _f, _f, _f, _f, _i, _i, _p],
+    "mig_ddpm_vlb_workspace_bytes": [_i, _l],
+    "mig_ddpm_vlb_term": [_i, _p, _p, _p, _p, _p, _l, _i, _i, _l, _i, _i, _f, _p, _p, _p, _l, _p],
     "mig_mse_fwd": [_i, _p, _p, _p, _p, _l, _i, _p],
     "mig_mse_bwd": [_i, _p, _p, _p, _p, _l, _i, _p],
     "mig_kl_fwd": [_i, _p, _p, _p, _p, _l, _i, _p],
@@ -111,7 +113,8 @@ _SIGNATURES = {
 }
 _RESTYPES = {"mig_last_error": C.c_char_p, "mig_conv_workspace_bytes": C.c_int64,
              "mig_groupnorm_workspace_bytes": C.c_int64, "mig_patch_stats_workspace_bytes": C.c_int64,
-             "mig_upconv_folded_elems": C.c_int64, "mig_ssim_workspace_bytes": C.c_int64}
+             "mig_upconv_folded_elems": C.c_int64, "mig_ssim_workspace_bytes": C.c_int64,
+             "mig_ddpm_vlb_workspace_bytes": C.c_int64}
 
 _lib = None
 

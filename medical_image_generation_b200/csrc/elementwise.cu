@@ -995,6 +995,168 @@ extern "C" int mig_ddim_step(int dtype, const void* model_out, const void* x, co
 }
 
 // ------------------------------------------------------------------------------------------------
+// DDPM variational bound (monai-generative DiffusionInferer.get_likelihood), one timestep per launch
+// ------------------------------------------------------------------------------------------------
+namespace mig {
+// Per-timestep scalars, one row of the fp32 table [T][kVlbCoefs] built on the host in upstream's operation order:
+// sqrt(acp_t), sqrt(1 - acp_t), c0, ct (the posterior-mean coefficients of `step` and `_get_mean`), the constant part
+// -1 + lv - lv + exp(lv - lv) of the KL of two Normals with the same log-variance lv, exp(-lv), exp(-0.5 lv).
+constexpr int kVlbCoefs = 7;
+// CTAs per launch (over all samples), fixed rather than derived from the SM count so that the workspace size and the
+// order of the reduction, hence the bits, depend only on (B, per_sample)
+constexpr int kVlbTargetCtas = 8 * 148;
+
+static int vlb_ctas_per_sample(int32_t B, int64_t per_sample) {
+  const int64_t want = (per_sample + 8 * 256 - 1) / (8 * 256);    // >= 8 elements per thread
+  const int64_t cap = (kVlbTargetCtas + B - 1) / B;
+  return (int)(want < 1 ? 1 : (want < cap ? want : cap));
+}
+
+struct VlbArgs {
+  const float* table;
+  int T, prediction, clip;
+  float half_bin, sqrt_2_over_pi;
+  int64_t per;
+  int vec;
+};
+
+// upstream's _approx_standard_normal_cdf: 0.5 (1 + tanh(sqrt(2/pi) (x + 0.044715 x^3))), every operation rounded as
+// the tensor expression rounds it (no contraction)
+__device__ __forceinline__ float vlb_cdf(float x, float k) {
+  const float x3 = __fmul_rn(__fmul_rn(x, x), x);
+  return __fmul_rn(0.5f, __fadd_rn(1.f, tanhf(__fmul_rn(k, __fadd_rn(x, __fmul_rn(0.044715f, x3))))));
+}
+
+// The bound term of one voxel: m the model output, xt the noisy sample, x0 the clean input, c the timestep's row
+__device__ __forceinline__ float vlb_voxel(float m, float xt, float x0, const float* c, bool decoder, const VlbArgs& a) {
+  const float sa = c[0], sb = c[1], c0 = c[2], ct = c[3];
+  float x0h;                                             // ddpm_step's expression
+  if (a.prediction == 0) x0h = (xt - sb * m) / sa;
+  else if (a.prediction == 1) x0h = m;
+  else x0h = sa * xt - sb * m;
+  if (a.clip) x0h = fminf(fmaxf(x0h, -1.f), 1.f);
+  const float ctx = __fmul_rn(ct, xt);
+  const float mu_p = __fadd_rn(__fmul_rn(c0, x0h), ctx);
+  if (!decoder) {                                        // KL(q(x_{t-1} | x_t, x_0) || p(x_{t-1} | x_t))
+    const float d = __fsub_rn(__fadd_rn(__fmul_rn(c0, x0), ctx), mu_p);
+    return __fmul_rn(0.5f, __fadd_rn(c[4], __fmul_rn(__fmul_rn(d, d), c[5])));
+  }
+  // -log p(x_0 | x_1): the discretised Gaussian of the decoder, log scale 0.5 lv, bins of the input quantisation
+  const float centered = __fsub_rn(x0, mu_p);
+  const float cdf_plus = vlb_cdf(__fmul_rn(c[6], __fadd_rn(centered, a.half_bin)), a.sqrt_2_over_pi);
+  const float cdf_min = vlb_cdf(__fmul_rn(c[6], __fsub_rn(centered, a.half_bin)), a.sqrt_2_over_pi);
+  float p;
+  if (x0 < -0.999f) p = cdf_plus;
+  else if (x0 > 0.999f) p = __fsub_rn(1.f, cdf_min);
+  else p = __fsub_rn(cdf_plus, cdf_min);
+  return -logf(fmaxf(p, 1e-12f));
+}
+
+// grid (gx, B): CTA (i, b) handles a grid-stride share of sample b, optionally stores its fp32 map, and writes the
+// fp64 sum of its share to partial[b * gx + i]
+template <typename T>
+__global__ void __launch_bounds__(256) ddpm_vlb_kernel(const T* __restrict__ m, const T* __restrict__ xt,
+                                                       const T* __restrict__ x0, const int64_t* __restrict__ ts,
+                                                       VlbArgs a, float* __restrict__ map,
+                                                       double* __restrict__ partial) {
+  constexpr int V = Vec16<T>::N;
+  __shared__ float coef[kVlbCoefs];
+  __shared__ double wsum[256 / 32];
+  const int b = blockIdx.y;
+  int64_t t = ts[b];
+  t = t < 0 ? 0 : (t >= a.T ? a.T - 1 : t);
+  if (threadIdx.x < kVlbCoefs) coef[threadIdx.x] = a.table[t * kVlbCoefs + threadIdx.x];
+  __syncthreads();
+  float c[kVlbCoefs];
+#pragma unroll
+  for (int q = 0; q < kVlbCoefs; ++q) c[q] = coef[q];
+  const bool decoder = t == 0;
+  const int64_t off = (int64_t)b * a.per;
+  const T *ms = m + off, *xs = xt + off, *zs = x0 + off;
+  float* mp = map ? map + off : nullptr;
+  const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+  const int64_t nvec = a.vec ? a.per / V : 0;
+  double acc = 0.0;
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < nvec; i += stride) {
+    Vec16<T> vm = ld16_stream(ms + i * V), vx = ld16_stream(xs + i * V), vz = ld16_stream(zs + i * V);
+    float kl[V], vsum = 0.f;
+#pragma unroll
+    for (int j = 0; j < V; ++j) {
+      kl[j] = vlb_voxel(vm.get(j), vx.get(j), vz.get(j), c, decoder, a);
+      vsum += kl[j];
+    }
+    acc += (double)vsum;   // one fp64 add per vector: the conversion and add per element cost bf16 throughput
+    if (mp) {
+#pragma unroll
+      for (int q = 0; q < V / 4; ++q)
+        reinterpret_cast<float4*>(mp + i * V)[q] = make_float4(kl[4 * q], kl[4 * q + 1], kl[4 * q + 2], kl[4 * q + 3]);
+    }
+  }
+  for (int64_t i = nvec * V + (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < a.per; i += stride) {
+    const float kl = vlb_voxel(to_f(ms[i]), to_f(xs[i]), to_f(zs[i]), c, decoder, a);
+    acc += (double)kl;
+    if (mp) mp[i] = kl;
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
+  if ((threadIdx.x & 31) == 0) wsum[threadIdx.x >> 5] = acc;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    double s = 0.0;
+    for (int w = 0; w < 256 / 32; ++w) s += wsum[w];
+    partial[(int64_t)b * gridDim.x + blockIdx.x] = s;
+  }
+}
+
+// total[b] += (sum of sample b's gx partials, added in a fixed order) / per_sample; one warp per sample
+__global__ void __launch_bounds__(256) ddpm_vlb_finish_kernel(const double* __restrict__ partial, int gx,
+                                                              double count, double* __restrict__ total, int B) {
+  const int b = (int)(((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5), lane = threadIdx.x & 31;
+  if (b >= B) return;
+  double s = 0.0;
+  for (int e = lane; e < gx; e += 32) s += partial[(int64_t)b * gx + e];
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+  if (lane == 0) total[b] += s / count;
+}
+}  // namespace mig
+
+extern "C" int64_t mig_ddpm_vlb_workspace_bytes(int32_t B, int64_t per_sample) {
+  if (B <= 0 || B >= 65536 || per_sample <= 0) return -1;
+  return (int64_t)B * vlb_ctas_per_sample(B, per_sample) * (int64_t)sizeof(double);
+}
+
+extern "C" int mig_ddpm_vlb_term(int dtype, const void* model_out, const void* x_t, const void* x0,
+                                 const int64_t* timesteps, const float* table, int64_t table_len, int32_t T,
+                                 int32_t B, int64_t per_sample, int prediction, int clip, float half_bin, float* kl_map,
+                                 double* total, void* workspace, int64_t workspace_bytes, void* stream) {
+  MIG_REQUIRE(B > 0 && B < 65536, "ddpm_vlb_term: batch must be in [1, 65535], got %d", (int)B);
+  MIG_REQUIRE(per_sample > 0, "ddpm_vlb_term: a sample must have at least one element");
+  MIG_REQUIRE(T > 0 && table_len == (int64_t)T * kVlbCoefs,
+              "ddpm_vlb_term: the coefficient table has %lld floats, expected %d timesteps x %d", (long long)table_len,
+              (int)T, kVlbCoefs);
+  MIG_REQUIRE(prediction >= 0 && prediction <= 2, "ddpm_vlb_term: prediction must be 0, 1 or 2");
+  MIG_REQUIRE(half_bin >= 0.f && half_bin < INFINITY, "ddpm_vlb_term: half bin width must be finite and >= 0");
+  MIG_REQUIRE(model_out && x_t && x0 && timesteps && table && total,
+              "ddpm_vlb_term: model_out, x_t, x0, timesteps, table and total must not be NULL");
+  const int gx = vlb_ctas_per_sample(B, per_sample);
+  const int64_t need = (int64_t)B * gx * (int64_t)sizeof(double);
+  MIG_REQUIRE(workspace && workspace_bytes >= need, "ddpm_vlb_term: workspace too small (%lld < %lld bytes)",
+              (long long)workspace_bytes, (long long)need);
+  VlbArgs a{table, T, prediction, clip, half_bin, sqrtf(0.636619772367581343f), per_sample, 0};
+  cudaStream_t st = as_stream(stream);
+  double* partial = (double*)workspace;
+  MIG_DISPATCH_DTYPE(dtype, TT, {
+    constexpr int V = Vec16<TT>::N;
+    a.vec = aligned16(model_out) && aligned16(x_t) && aligned16(x0) && aligned16(kl_map) && per_sample % V == 0;
+    ddpm_vlb_kernel<TT><<<dim3(gx, B), 256, 0, st>>>((const TT*)model_out, (const TT*)x_t, (const TT*)x0, timesteps, a,
+                                                     kl_map, partial);
+  });
+  ddpm_vlb_finish_kernel<<<(B + 7) / 8, 256, 0, st>>>(partial, gx, (double)per_sample, total, B);
+  return check_launch("ddpm_vlb_term");
+}
+
+// ------------------------------------------------------------------------------------------------
 // losses
 // ------------------------------------------------------------------------------------------------
 namespace mig {

@@ -5,6 +5,7 @@ from __future__ import annotations
 import torch
 
 from . import ops
+from .schedulers import DDPMScheduler
 
 
 class DiffusionInferer:
@@ -62,6 +63,68 @@ class DiffusionInferer:
                 intermediates.append(image)
         return (image, intermediates) if save_intermediates else image
 
+    @torch.no_grad()
+    def get_likelihood(self, inputs, diffusion_model, scheduler=None, save_intermediates: bool = False,
+                       conditioning=None, mode: str = "crossattn", original_input_range=(0, 255),
+                       scaled_input_range=(0, 1), verbose: bool = True, *, noise=None, cuda_graph: bool = False):
+        """The DDPM variational bound of each input, in nats per element: over `scheduler.timesteps`, the mean KL
+        between the posterior q(x_{t-1} | x_t, x_0) and the model's p(x_{t-1} | x_t), and at t = 0 the mean negative
+        log-likelihood of the input under the discretised Gaussian decoder whose bins are those of
+        `original_input_range` scaled to `scaled_input_range`. Returns the fp32 (B,) total on the inputs' device (summed
+        in fp64 on the device) and, with `save_intermediates`, the fp32 CPU map of every timestep.
+
+        As upstream, one noise tensor is drawn for all timesteps and x_t comes from `self.scheduler.add_noise`. Each
+        timestep's bound term is one fused kernel that reads its scalars from a device table, so `cuda_graph=True`
+        (extra, optional) captures add_noise, the model forward and the bound term once and replays the whole step.
+        `noise` (extra, optional) injects the noise for parity tests. `verbose` is accepted and ignored."""
+        scheduler = scheduler or self.scheduler
+        if not isinstance(scheduler, DDPMScheduler):
+            raise NotImplementedError(f"Likelihood computation is only compatible with DDPMScheduler, you are using "
+                                      f"{type(scheduler).__name__}")
+        if mode not in ("crossattn", "concat"):
+            raise NotImplementedError(f"{mode} condition is not supported")
+        ops._require_cuda(inputs, "get_likelihood")
+        B = inputs.shape[0]
+        noise = torch.randn_like(inputs) if noise is None else noise.to(device=inputs.device, dtype=inputs.dtype)
+        bin_width = (scaled_input_range[1] - scaled_input_range[0]) / (original_input_range[1] - original_input_range[0])
+        half_bin = bin_width / 2
+        total = torch.zeros(B, dtype=torch.float64, device=inputs.device)
+        workspace = scheduler._vlb_workspace(inputs)
+        intermediates = []
+
+        def step(tt, acc, kl_map=None):
+            """add_noise, the forward and the bound term of timestep tensor `tt`; adds into `acc`, returns the map."""
+            noisy = self.scheduler.add_noise(original_samples=inputs, noise=noise, timesteps=tt)
+            if mode == "concat":
+                out = diffusion_model(ops.cat_channels(noisy, conditioning), timesteps=tt, context=None)
+            else:
+                out = diffusion_model(x=noisy, timesteps=tt, context=conditioning)
+            m, x, x0 = scheduler._vlb_operands(out, noisy, inputs)
+            if save_intermediates and kl_map is None:
+                kl_map = torch.empty_like(x, dtype=torch.float32)
+            scheduler._vlb_term(m, tt, x, x0, acc, workspace, kl_map, half_bin)
+            return kl_map
+
+        graph = None
+        if cuda_graph and len(scheduler.timesteps) > 2:
+            static_t = torch.full((B,), int(scheduler.timesteps[0]), dtype=torch.int64, device=inputs.device)
+            static_map = step(static_t, torch.zeros_like(total))   # warm-up: workspaces, filter shadows, tensor maps
+            torch.cuda.synchronize()
+            graph = torch.cuda.CUDAGraph()
+            with torch.cuda.graph(graph):
+                step(static_t, total, static_map)
+        for t in scheduler.timesteps:
+            if graph is not None:
+                static_t.fill_(int(t))
+                graph.replay()
+                kl_map = static_map
+            else:
+                kl_map = step(torch.full((B,), int(t), dtype=torch.int64, device=inputs.device), total)
+            if save_intermediates:
+                intermediates.append(kl_map.cpu())
+        total = total.float()
+        return (total, intermediates) if save_intermediates else total
+
 
 class LatentDiffusionInferer(DiffusionInferer):
     def __init__(self, scheduler, scale_factor: float = 1.0) -> None:
@@ -87,3 +150,27 @@ class LatentDiffusionInferer(DiffusionInferer):
             return image, [autoencoder_model.decode_stage_2_outputs(ops.scale(l, 1.0 / float(self.scale_factor)))
                            for l in inter]
         return image
+
+    @torch.no_grad()
+    def get_likelihood(self, inputs, autoencoder_model, diffusion_model, scheduler=None,
+                       save_intermediates: bool = False, conditioning=None, mode: str = "crossattn",
+                       original_input_range=(0, 255), scaled_input_range=(0, 1), verbose: bool = True,
+                       resample_latent_likelihoods: bool = False, resample_interpolation_mode: str = "nearest", *,
+                       noise=None, cuda_graph: bool = False):
+        """`DiffusionInferer.get_likelihood` of the latents `encode_stage_2_inputs(inputs) * scale_factor`. With
+        `resample_latent_likelihoods` (which needs `save_intermediates`), every latent map is resized to the inputs'
+        spatial shape with `nn.Upsample(mode=resample_interpolation_mode)`, as upstream does on its CPU maps."""
+        if resample_latent_likelihoods and not save_intermediates:
+            raise ValueError(f"If `resample_latent_likelihoods` is True, `save_intermediates` must also be True, got "
+                             f"{save_intermediates}")
+        if resample_latent_likelihoods and resample_interpolation_mode not in ("nearest", "bilinear", "trilinear"):
+            raise ValueError(f"resample_interpolation_mode should be either nearest, bilinear, or trilinear, got "
+                             f"{resample_interpolation_mode}")
+        latents = ops.scale(autoencoder_model.encode_stage_2_inputs(inputs), float(self.scale_factor))
+        out = super().get_likelihood(latents, diffusion_model, scheduler, save_intermediates, conditioning, mode,
+                                     original_input_range, scaled_input_range, verbose, noise=noise,
+                                     cuda_graph=cuda_graph)
+        if save_intermediates and resample_latent_likelihoods:
+            resizer = torch.nn.Upsample(size=tuple(inputs.shape[2:]), mode=resample_interpolation_mode)
+            out = (out[0], [resizer(m) for m in out[1]])
+        return out

@@ -5,6 +5,8 @@ train_ddpm.py:380-382), backed by fused sm_100a kernels:
   add_noise / get_velocity      : one 128-bit vectorised kernel, per-sample coefficient gather (K14)
   DDPMScheduler.step            : ONE kernel per reverse step instead of ~12 elementwise launches (K15)
   DDIMScheduler.step / reversed_step : ONE kernel per step (ddim_step), for few-step sampling and DDIM inversion
+  DDPMScheduler._vlb_term       : ONE kernel per timestep of the likelihood bound (ddpm_vlb_term), scalars from a device
+                                  table (`vlb_coefficients`) so the whole timestep can be graph-captured
 
 Index arithmetic (timesteps, alpha_bar[t], alpha_bar[t-1]) is done exactly as upstream: fp32 tables built
 with torch on the host, `set_timesteps` in numpy int64, per-step coefficients evaluated in fp32 on the
@@ -18,7 +20,7 @@ import numpy as np
 import torch
 
 from . import ops
-from ._lib import call
+from ._lib import call, load
 
 
 def _betas(schedule: str, num_train_timesteps: int, beta_start: float = 1e-4, beta_end: float = 2e-2,
@@ -146,16 +148,83 @@ class DDPMScheduler(_NoiseSchedule):
         beta_prod_prev = 1 - acp_prev
         c0 = (acp_prev ** 0.5 * self.betas[t]) / beta_prod_t
         ct = self.alphas[t] ** 0.5 * beta_prod_prev / beta_prod_t
-        sigma = torch.tensor(0.0)
-        if t > 0:
-            var = (1 - acp_prev) / (1 - acp_t) * self.betas[t]
-            if self.variance_type == "fixed_small":
-                var = torch.clamp(var, min=1e-20)
-            elif self.variance_type == "fixed_large":
-                var = self.betas[t]
-            sigma = var ** 0.5
+        sigma = self._get_variance(t) ** 0.5 if t > 0 else torch.tensor(0.0)
         return dict(sqrt_acp=float(acp_t ** 0.5), sqrt_one_minus_acp=float(beta_prod_t ** 0.5), c0=float(c0),
                     ct=float(ct), sigma=float(sigma), t=t, t_prev=t - 1)
+
+    def _get_variance(self, timestep: int) -> torch.Tensor:
+        """The fp32 variance of the posterior step at `timestep` (upstream `_get_variance`, fixed variance types)."""
+        t = int(timestep)
+        acp_t = self.alphas_cumprod[t]
+        acp_prev = self.alphas_cumprod[t - 1] if t > 0 else self.one
+        var = (1 - acp_prev) / (1 - acp_t) * self.betas[t]
+        if self.variance_type == "fixed_small":
+            var = torch.clamp(var, min=1e-20)
+        elif self.variance_type == "fixed_large":
+            var = self.betas[t]
+        return var
+
+    # -- likelihood ------------------------------------------------------------------------------------
+    VLB_COEFS = ("sqrt_acp", "sqrt_one_minus_acp", "c0", "ct", "kl_const", "inv_var", "inv_std")
+
+    def vlb_coefficients(self) -> torch.Tensor:
+        """(T, 7) fp32 CPU table of the per-timestep scalars of the variational bound, evaluated like upstream
+        `get_likelihood` evaluates them: the coefficients of `step`, and with lv = log(variance) the constant part of
+        the KL of two Normals of equal variance (-1 + lv - lv + exp(lv - lv)), exp(-lv) and exp(-0.5 lv)."""
+        rows = []
+        for t in range(self.num_train_timesteps):
+            k = self.step_coefficients(t)
+            lv = torch.log(self._get_variance(t))
+            kl_const = -1.0 + lv - lv + torch.exp(lv - lv)
+            rows.append([k["sqrt_acp"], k["sqrt_one_minus_acp"], k["c0"], k["ct"], float(kl_const),
+                         float(torch.exp(-lv)), float(torch.exp(-(0.5 * lv)))])
+        return torch.tensor(rows, dtype=torch.float32)
+
+    def _vlb_table_on(self, device) -> torch.Tensor:
+        key = ("vlb", self.variance_type, device)
+        t = self._dev_tables.get(key)
+        if t is None:
+            t = self.vlb_coefficients().to(device).contiguous()
+            self._dev_tables[key] = t
+        return t
+
+    def _vlb_workspace(self, sample) -> torch.Tensor:
+        """A scratch buffer large enough for `_vlb_term` on samples shaped like `sample`."""
+        B = sample.shape[0]
+        nbytes = load().mig_ddpm_vlb_workspace_bytes(B, sample.numel() // max(B, 1))
+        if nbytes < 0:
+            raise RuntimeError(f"_vlb_term: no workspace for a batch of shape {tuple(sample.shape)}")
+        return torch.empty(nbytes, dtype=torch.uint8, device=sample.device)
+
+    def _vlb_term(self, model_output, timesteps, sample, original_samples, total, workspace, kl_map=None,
+                 half_bin: float = 0.5 / 255):
+        """One timestep of upstream `get_likelihood` in one launch: the KL term (t > 0) or the decoder negative
+        log-likelihood (t == 0) of every element, from the model output at the noisy `sample` x_t and the clean
+        `original_samples` x_0, t per sample from the device tensor `timesteps`. Adds each sample's mean into `total`
+        (fp64 (B,), on the device) and writes the fp32 map into `kl_map` when given (shaped and strided like the
+        operands as returned by `_vlb_operands`). `half_bin` is half the decoder's bin width."""
+        B = sample.shape[0]
+        if timesteps.dtype != torch.int64 or timesteps.numel() != B or not timesteps.is_contiguous():
+            raise RuntimeError(f"vlb_term: timesteps must be {B} contiguous int64 values")
+        if total.dtype != torch.float64 or total.numel() != B:
+            raise RuntimeError(f"vlb_term: total must hold {B} float64 values")
+        if kl_map is not None and (kl_map.dtype != torch.float32 or kl_map.stride() != sample.stride()
+                                   or kl_map.shape != sample.shape):
+            raise RuntimeError("vlb_term: kl_map must be float32, shaped and strided like the sample")
+        table = self._vlb_table_on(sample.device)
+        call("mig_ddpm_vlb_term", ops._dt(sample), ops._ptr(model_output), ops._ptr(sample), ops._ptr(original_samples),
+             ops._ptr(timesteps), ops._ptr(table), table.numel(), self.num_train_timesteps, B, sample.numel() // B,
+             _PREDICTION[self.prediction_type], int(self.clip_sample), float(half_bin), ops._ptr(kl_map),
+             ops._ptr(total), ops._ptr(workspace), workspace.numel(), ops._stream())
+
+    def _vlb_operands(self, model_output, sample, original_samples):
+        """(m, x_t, x_0) in one dtype (float32 or bfloat16, the sample's) and one layout (contiguous or channels-last,
+        the sample's when both others can take it; otherwise all contiguous)."""
+        x, m = self._step_operands(model_output, sample)
+        x0 = original_samples.to(x.dtype)
+        if x0.stride() != x.stride():
+            x, m, x0 = x.contiguous(), m.contiguous(), x0.contiguous()
+        return m, x, x0
 
     def step(self, model_output, timestep, sample, generator=None, noise=None):
         """One reverse-diffusion step. Returns (pred_prev_sample, pred_original_sample).
