@@ -722,7 +722,8 @@ static bool pick_box(int D, int H, int W, int* bd, int* bh, int* bw) {
                                 {1, 1, 64}, {8, 4, 2}, {4, 8, 2}, {16, 2, 2}, {2, 16, 2}, {8, 8, 1}, {16, 4, 1},
                                 {4, 16, 1}};
   // Boxes may overhang the tensor (TMA zero-fills out-of-bounds voxels, the epilogue masks them): pick the shape
-  // that wastes the fewest rows; exact tilings (efficiency 1) win, e.g. 24^3 -> 1x8x8, 12^3 -> 4x4x4, 6^3 -> 2x4x8.
+  // that wastes the fewest rows; exact tilings (efficiency 1) win, e.g. 24^3 -> 1x8x8, 12^3 -> 4x4x4. On a tie the
+  // earlier candidate wins: 6^3 -> 1x8x8 (2x4x8 wastes as many rows).
   double best = 0.0;
   for (auto& c : cand) {
     const double cover = (double)((D + c[0] - 1) / c[0] * c[0]) * ((H + c[1] - 1) / c[1] * c[1]) *
@@ -737,7 +738,7 @@ static bool pick_box(int D, int H, int W, int* bd, int* bh, int* bw) {
 }
 
 // wgrad: a box is one K stage, so its voxel count only has to be a multiple of 16 (the UMMA K). Besides the 64-voxel
-// shapes, 48/32/16-voxel boxes are tried for volumes the 64-voxel boxes tile badly (6^3: 4x2x6 boxes, 75 % instead of
+// shapes, 48/32/16-voxel boxes are tried for volumes the 64-voxel boxes tile badly (6^3: 2x4x6 boxes, 75 % instead of
 // 56 % useful rows); smaller stages pay relatively more per-stage overhead, hence the discount.
 static bool pick_box_k(int D, int H, int W, int* bd, int* bh, int* bw) {
   bool ok = pick_box(D, H, W, bd, bh, bw);

@@ -45,7 +45,7 @@ CONV_CASES = [
     (1, 64, 24, (8, 8, 8), (3, 3, 3), (1, 1, 1), (1, 1, 1)),      # narrow output (BN = 32), dgrad falls back (Cout % 64)
     (8, 64, 256, (24, 24, 24), (3, 3, 3), (1, 1, 1), (1, 1, 1)),  # BASELINE-size level 0: fwd uses the 256x256 CTA tile
     (8, 256, 64, (24, 24, 24), (3, 3, 3), (1, 1, 1), (1, 1, 1)),  # ... and dgrad / wgrad use it here
-    (2, 128, 256, (6, 6, 6), (3, 3, 3), (1, 1, 1), (1, 1, 1)),    # 6^3: overhanging 2x4x8 boxes, split-K
+    (2, 128, 256, (6, 6, 6), (3, 3, 3), (1, 1, 1), (1, 1, 1)),    # 6^3: 3x6x6 boxes in 128-row slots, split-K
     (3, 64, 64, (6, 6, 6), (3, 3, 3), (1, 1, 1), (1, 1, 1)),      # 6^3: 3x6x6 boxes in 128-row slots (108 valid rows), odd box count
     (2, 64, 128, (5, 5, 5), (3, 3, 3), (1, 1, 1), (1, 1, 1)),     # 5^3: one 125-row box per sample
     (1, 64, 3, (8, 8, 8), (3, 3, 3), (1, 1, 1), (1, 1, 1)),       # out conv of the LDM U-Net: 3 output channels on the TMA kernel
